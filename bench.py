@@ -2,7 +2,7 @@
 """
 bench.py -- measures the hot path on B200 (contract: one JSON line on stdout from rank 0).
 
-  python bench.py --gpus N --steps K --warmup W [--workload x|self|map|cov|c5] [--impl b200|reference]
+  python bench.py --gpus N --steps K --warmup W [--workload x|self|map|cov|c5] [--impl b200|reference] [--dump-outputs DIR]
 
 Default workload = BASELINE config 4 (`mimeo x`, 50 Mbp vs 100 Mbp), the largest named config that fits one GPU within the
 driver's time and the one BASELINE.json shards over 8 GPUs; the same job at every N (strong scaling). Configs 1, 2 and 3 are
@@ -64,6 +64,25 @@ def ncu_pipes(workload, kernel):
             return json.load(f)[workload][kernel].get('pipes')
     except Exception:
         return None
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy in float64 (every int32 coordinate, score and count is exact there), at
+    most DUMP_BYTES in all. An array larger than its share of what is left keeps a sample of its rows drawn with a fixed
+    seed, in their original order, so two builds run with the same arguments write comparable files."""
+    os.makedirs(out_dir, exist_ok=True)
+    budget = DUMP_BYTES - 4096 * len(arrays)                 # room for the .npy headers
+    items = sorted(((k, np.asarray(v, dtype=np.float64)) for k, v in arrays.items()), key=lambda kv: kv[1].nbytes)
+    for i, (name, a) in enumerate(items):
+        share = budget // (len(items) - i)
+        if a.nbytes > share:
+            keep = share // (a.nbytes // len(a))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+        budget -= a.nbytes
 
 
 class ClockSampler:
@@ -131,6 +150,10 @@ class CoverageWorkload:
         out = coverage.coverage_segments_device(self.dev[0], self.dev[1], self.dev[2], self.sizes, self.MIN_COV, self.MIN_LEN)
         self.nseg = int(out[0].numel())
         return out
+
+    def outputs(self, out):
+        """What a caller of step_resident receives: the (scaffold, start, end) segments as one [n, 3] array."""
+        return {'segments': np.stack([t.cpu().numpy() for t in out], axis=1)}
 
     def step_e2e(self):
         from mimeo_b200 import coverage
@@ -270,6 +293,14 @@ class AlignWorkload:
 
     def step_resident(self):
         return self._annotate(self._align_filter(self.T, self.Q, self.Qb))
+
+    def outputs(self, out):
+        """What a caller of step_resident receives on rank 0: the filtered hit table [n, 10] (columns HIT_FIELDS, global
+        scaffold ids) and the segments [m, 3] of every coverage pass."""
+        if out is None:
+            return {}
+        table, segs = out
+        return {'hits': table, **{f'segments_{name}': v for name, v in segs.items()}}
 
     def step_e2e(self):
         """Host ASCII (pinned) in -> .tab rows and GFF3 rows out on rank 0, every copy and the collectives inside."""
@@ -534,12 +565,13 @@ def run_b200(args):
     barrier()
     total_ms = 0.0
     for _ in range(args.steps):
+        out = None                          # free the previous step's result first: the step reuses its device buffers
         flush.zero_()                       # L2 flush between timed iterations (outside the timed interval)
         barrier()                           # every rank starts the step together: the step contains collectives
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         with torch.cuda.stream(stream):
             e0.record(stream)
-            wl.step_resident()
+            out = wl.step_resident()
             e1.record(stream)
         e1.synchronize()
         total_ms += e0.elapsed_time(e1)
@@ -638,9 +670,9 @@ def run_b200(args):
 
     # ---- the other single-GPU BASELINE configs beside the headline (default workload, 1 GPU only): extra keys, never mixed into `value`
     if rank == 0 and world == 1 and args.workload == DEFAULT_WORKLOAD and not os.environ.get('MB2_BENCH_NO_SIDE'):
-        for key, w, st in (('config1_self_5Mbp', 'self', 5), ('config2_coverage_stage', 'cov', 5), ('config3_map_40Mbp', 'map', 3)):
+        for key, w in (('config1_self_5Mbp', 'self'), ('config2_coverage_stage', 'cov'), ('config3_map_40Mbp', 'map')):
             try:
-                extra[key] = side_config(w, steps=st)
+                extra[key] = side_config(w, steps=args.steps, warmup=args.warmup)
             except Exception as e:      # the headline line must not depend on these legs
                 extra[key] = {'error': f'{type(e).__name__}: {e}'[:300]}
 
@@ -664,6 +696,8 @@ def run_b200(args):
             ok, nrows = wl.parity(rows, pairs)
             parity = {'rows_identical': bool(ok), 'rows_compared': nrows, 'pairs_compared': len(pairs),
                       'scope': 'every alignment row (t, q, strand, start1, end1, start2+, end2+, score, matches, columns) of the sampled scaffold pairs, GPU vs oracle'}
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, wl.outputs(out))
 
     sys.stdout.flush()
     os.dup2(saved_stdout, 1)
@@ -693,7 +727,13 @@ def main():
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--workload', default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
     ap.add_argument('--ref-pairs', type=int, default=0, help='reference arm: scaffold pairs per step (default 2 x host cores)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write what the last timed step returned on rank 0 as DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes what the GPU path computed; the reference arm keeps no outputs')
     args.warmup = max(args.warmup, 3) if args.impl == 'b200' else args.warmup
     if args.impl == 'reference':
         run_reference(args)
