@@ -125,6 +125,15 @@ __device__ __forceinline__ void xdrop_window30(uint32_t tab_sa, uint32_t m10, ui
     nchunks += (uint32_t)entered - (parked >> 24);
     if (slow) D = d_keep;
 }
+// (best, D) of one side in a deferred record: best < 2^16 (at most 90 columns of at most +100), an open D < 2^13 (the min
+// field); a terminated side stores 0xFFFF in the D half.
+__device__ __forceinline__ uint32_t s1_pack(int best, int D) {
+    return (uint32_t)best | ((D < S1_DONE / 2 ? (uint32_t)D : 0xFFFFu) << 16);
+}
+__device__ __forceinline__ void s1_unpack(uint32_t w, int& best, int& D) {
+    best = (int)(w & 0xFFFFu);
+    D = (w >> 16) == 0xFFFFu ? S1_DONE : (int)(w >> 16);
+}
 
 // 128 columns of one sequence in registers, starting at the 64-column boundary at or below `first`: packed bases, non-ACGT
 // flags and (when the genome is soft-masked) the not-seedable flags.
@@ -176,6 +185,21 @@ __device__ __forceinline__ SeqBlock load_block(const uint64_t* __restrict__ pk, 
     return b;
 }
 
+// Appends the survivors of a warp (diagonal, query position) at one atomically reserved range of surv.
+__device__ __forceinline__ void append_survivors(bool survivor, uint32_t hi, uint32_t hj, uint32_t diag_bias, int lane,
+                                                 uint64_t* __restrict__ surv, uint32_t surv_cap, unsigned long long* __restrict__ counters) {
+    const uint32_t smask = __ballot_sync(0xffffffffu, survivor);
+    if (smask) {
+        unsigned long long basev = 0;
+        if (lane == __ffs(smask) - 1) basev = atomicAdd(&counters[0], (unsigned long long)__popc(smask));
+        basev = __shfl_sync(0xffffffffu, basev, __ffs(smask) - 1);
+        if (survivor) {
+            const unsigned long long slot = basev + __popc(smask & ((1u << lane) - 1u));
+            if (slot < surv_cap) surv[slot] = ((uint64_t)(hi - hj + diag_bias) << 32) | hj;
+        }
+    }
+}
+
 // ---- load-balanced scan --------------------------------------------------------------------------------------
 // Every WARP works on its own: no CTA barrier after the table build. A warp takes 32 consecutive query positions per
 // round (lane = position); rounds are handed out by an atomic counter. Phase A: the 13 bucket ranges of each position are looked up, the non-empty ones are
@@ -185,6 +209,12 @@ __device__ __forceinline__ SeqBlock load_block(const uint64_t* __restrict__ pk, 
 // (30-column windows, 3 columns per table lookup). Leftover hits (< 32) wait for the next round, so batches are always
 // full except for the very last one of a warp. All loads of a batch that do not depend on the x-drop outcome (leader
 // windows, first right and left windows) are issued together.
+// A batch runs right window 0 and left windows 0 and 1. Right window 1 (needed by about 12 % of random hits, but by some lane
+// of almost every batch) and left window 2 (about 2.5 %) would cost the whole warp for a few lanes, so a hit that is still
+// open on the right after window 0 or on the left after window 1 is deferred instead: its state
+// (target and query position, (best, D) of both sides) goes to the warp's queue of deferred hits, and whenever 32 are queued
+// (and once more at the end of the warp's work) a drain batch resumes them, one per lane, where their batch left them.
+// Which hits survive and how many chunks each enters do not depend on which lanes share a warp.
 constexpr int SC_NT = 256;                 // threads per CTA
 constexpr int SC_WARPS = SC_NT / 32;
 constexpr int SC_NPROBE = 13;
@@ -192,6 +222,24 @@ constexpr int SC_HALF = 3;                 // probes appended per step: at most 
 constexpr int SC_STEPS = (SC_NPROBE + SC_HALF - 1) / SC_HALF;   // steps per round
 constexpr int SC_RING = 128;               // descriptors per warp: < 32 pending (every descriptor holds >= 1 hit) + 96 new
                                            // (a small ring keeps shared memory low, which leaves the SM more L1 for the gathers)
+constexpr int SC_DQ = 64;                  // deferred hits per warp: < 32 queued (drained at 32) + at most 32 from one batch
+
+// Window b >= 1 of the right or the left side of hit (hi, hj) in extension order (the left side reversed), for a lane whose
+// side is still open (D); zero columns (a no-op) otherwise.
+__device__ __forceinline__ void s1_later_window(const GenomeView& T, const GenomeView& Q, uint32_t hi, uint32_t hj, bool right, int b, int D,
+                                                uint64_t& wt, uint64_t& wq, uint32_t& an) {
+    wt = 0; wq = 0; an = 0;
+    if (D >= S1_DONE / 2) return;
+    if (right) {
+        const uint32_t ct = hi + SEED_SPAN + S1_WINDOW * b, cq = hj + SEED_SPAN + S1_WINDOW * b;
+        wt = window32(T.pk, ct); wq = window32(Q.pk, cq);
+        an = (nwindow32(T.nm, ct) | nwindow32(Q.nm, cq)) & S1_WINDOW_MASK;
+    } else {
+        const uint32_t ct = hi + SEED_SPAN - S1_WINDOW * b - 32, cq = hj + SEED_SPAN - S1_WINDOW * b - 32;
+        wt = rev2groups(window32(T.pk, ct)); wq = rev2groups(window32(Q.pk, cq));
+        an = __brev(nwindow32(T.nm, ct) | nwindow32(Q.nm, cq)) & S1_WINDOW_MASK;
+    }
+}
 
 template <int MINB, uint32_t TAILVOTES>
 __global__ void __launch_bounds__(SC_NT, MINB)
@@ -200,6 +248,7 @@ seed_scan_kernel(GenomeView T, GenomeView Q, const uint32_t* __restrict__ off, c
                  uint64_t* __restrict__ surv, uint32_t surv_cap, unsigned long long* __restrict__ counters) {
     __shared__ uint32_t s1tab[S1_TAB];
     __shared__ uint32_t r_cum[SC_WARPS][SC_RING], r_b0[SC_WARPS][SC_RING], r_j[SC_WARPS][SC_RING];
+    __shared__ uint4 r_defer[SC_WARPS][SC_DQ];     // deferred hits {hi, hj, s1_pack(right), s1_pack(left)}
     __shared__ unsigned long long sh_stat[3];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (int e = tid; e < S1_TAB; e += SC_NT) s1tab[e] = s1_entry((uint32_t)e, X);
@@ -210,6 +259,7 @@ seed_scan_kernel(GenomeView T, GenomeView Q, const uint32_t* __restrict__ off, c
     uint32_t* __restrict__ rc = r_cum[warp];
     uint32_t* __restrict__ rb = r_b0[warp];
     uint32_t* __restrict__ rj = r_j[warp];
+    uint4* __restrict__ dq = r_defer[warp];
     const int nprobe = transition ? SC_NPROBE : 1;
     const uint32_t nrounds = (q_n + 31) / 32;
     // Rounds are handed out dynamically (counters[CNT_WORK], zeroed by the caller): hits per round vary by orders of magnitude
@@ -221,6 +271,7 @@ seed_scan_kernel(GenomeView T, GenomeView Q, const uint32_t* __restrict__ off, c
     bool exhausted = false;
     uint32_t head = 0, tail = 0;            // ring positions (monotone, used modulo SC_RING)
     uint32_t cum_tail = 0, consumed = 0;    // hits appended / processed so far (wrapping arithmetic)
+    uint32_t dq_head = 0, dq_tail = 0;      // deferred hits drained / queued so far (monotone, used modulo SC_DQ)
     unsigned long long n_lead = 0, n_cells = 0, n_hits = 0;
     for (;;) {
         // ---------------- phase A: append half rounds until a full batch is pending
@@ -273,102 +324,106 @@ seed_scan_kernel(GenomeView T, GenomeView Q, const uint32_t* __restrict__ off, c
             tail += tot_n; cum_tail += tot_h; n_hits += (lane == 0) ? tot_h : 0;
             __syncwarp();
         }
-        const uint32_t pending = cum_tail - consumed;
-        if (pending == 0) break;
-        // ---------------- phase B: one batch of up to 32 hits, one per lane
-        const uint32_t nb = min(pending, 32u);
-        bool live = (uint32_t)lane < nb;
-        const uint32_t h = consumed + (uint32_t)lane;
-        uint32_t hi = 0, hj = 0, e_last = head;
-        {
-            // Descriptor of every hit of the batch without a search: rc[head] <= consumed < rc[head + 1] (invariant of `head`) and
-            // every descriptor holds at least one hit, so the batch lies inside descriptors head .. head + 31. Lane i looks at
-            // descriptor head + i; the ones that START inside the batch (at offset 1..31) set a bit at their offset; the
-            // descriptor of the hit at offset l is head + (bits at or below l).
-            const uint32_t di = head + (uint32_t)lane;
-            const bool dv = (int32_t)(tail - di) > 0;
-            const uint32_t ci = dv ? rc[di & (SC_RING - 1)] : 0u;
-            const uint32_t first = ci - consumed;                   // wrapping; >= 1 for lane > 0
-            const uint32_t starts = __reduce_or_sync(0xffffffffu, (dv && lane > 0 && first < 32u) ? (1u << first) : 0u);
+        const uint32_t pending = cum_tail - consumed, queued = dq_tail - dq_head;
+        if (pending == 0 && queued == 0) break;
+        uint32_t hi = 0, hj = 0, nchunks = 0;
+        int best_r = 0, dr = S1_DONE, best_l = 0, dl = S1_DONE;
+        bool live;
+        if (queued >= 32u || pending == 0) {
+            // ---------------- drain: up to 32 deferred hits, one per lane, resume from their stored (best, D)
+            static_assert(S1_RIGHT_WINDOWS == 2 && S1_LEFT_WINDOWS == 3, "a batch runs right window 0 and left windows 0, 1; a drain the rest");
+            const uint32_t nd = min(queued, 32u);
+            live = (uint32_t)lane < nd;
             if (live) {
-                const uint32_t lo = head + (uint32_t)__popc(starts & ((2u << lane) - 1u));
-                e_last = lo;
-                hi = pos[rb[lo & (SC_RING - 1)] + (h - rc[lo & (SC_RING - 1)])];
-                hj = rj[lo & (SC_RING - 1)];
+                const uint4 r = dq[(dq_head + (uint32_t)lane) & (SC_DQ - 1)];
+                hi = r.x; hj = r.y;
+                s1_unpack(r.z, best_r, dr);
+                s1_unpack(r.w, best_l, dl);
             }
-        }
-        // Everything the batch needs that does not depend on the x-drop outcome: leader window (p - 1), first right window
-        // (p + 19) and first left window (p - 13). All three lie inside the 128 columns that start at the 64-column boundary
-        // below p - 13, so each sequence is fetched as ONE aligned block (32 bytes of packed bases, 16 of flags: four load
-        // instructions per sequence instead of twelve) and the windows are cut out of registers. After the bank fix of the
-        // extension table (xdrop_table.cuh) the scan is bound by the integer ALU pipe (ncu on C4: alu pipe 74 % busy, L1 data
-        // pipe 65 %, DRAM 11 %; profiles/r2_seed_scan_c4_v2_ncu_summary.txt); taking the pos[] and target gathers of the next
-        // batch off the critical path (a pipelined variant, measured) changed nothing and was dropped.
-        uint64_t lt = 0, lq = 0, rt = 0, rq = 0, ft = 0, fq = 0;
-        uint32_t ln = 1, rn = 0, fn = 0;
-        if (live) {
-            const SeqBlock bt = load_block(T.pk, T.nm, T.sm, hi - 13), bq = load_block(Q.pk, Q.nm, Q.sm, hj - 13);
-            uint32_t tfn, trn, tls, qfn, qrn, qls;
-            bt.windows(hi - 13, ft, lt, rt, tfn, trn, tls);
-            bq.windows(hj - 13, fq, lq, rq, qfn, qrn, qls);
-            ln = (tls | qls) & SEED_WINDOW_MASK19;
-            rn = (trn | qrn) & S1_WINDOW_MASK;
-            fn = __brev(tfn | qfn) & S1_WINDOW_MASK;
-            // spec D1: only run leaders are candidates
-            if (ln == 0 && seed_match(lt, lq, transition != 0)) live = false; else n_lead++;
-        }
-        // Right of the seed: up to S1_RIGHT_WINDOWS windows of 30 columns. Left, from the last seed column downwards: up to
-        // S1_LEFT_WINDOWS windows, reversed so that the same forward-order table applies. The first window of either side comes
-        // out of the blocks above and runs without polling (some lane of 32 is practically always still open at its end; on the
-        // left its first 19 columns are the seed itself); in the later windows a warp leaves as soon as all its lanes are done.
-        const int d_start = live ? S1_D0 : S1_DONE;
-        int best_r = 0, dr = d_start;
-        uint32_t nchunks = 0;
-        xdrop_window30<0u>(s1tab_sa, s1_m10, s1_m9, rt, rq, rn, X, best_r, dr, nchunks);
-#pragma unroll 1
-        for (int b = 1; b < S1_RIGHT_WINDOWS; b++) {
-            if (__all_sync(0xffffffffu, dr >= S1_DONE / 2)) break;
-            uint64_t wt = 0, wq = 0; uint32_t an = 0;
-            if (dr < S1_DONE / 2) {
-                const uint32_t ct = hi + SEED_SPAN + S1_WINDOW * b, cq = hj + SEED_SPAN + S1_WINDOW * b;
-                wt = window32(T.pk, ct); wq = window32(Q.pk, cq);
-                an = (nwindow32(T.nm, ct) | nwindow32(Q.nm, cq)) & S1_WINDOW_MASK;
+            dq_head += nd;
+            uint64_t wt, wq; uint32_t an;
+            if (!__all_sync(0xffffffffu, dr >= S1_DONE / 2)) {
+                s1_later_window(T, Q, hi, hj, true, 1, dr, wt, wq, an);
+                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, wt, wq, an, X, best_r, dr, nchunks);
             }
-            xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, wt, wq, an, X, best_r, dr, nchunks);
-        }
-        const bool open_r = dr < S1_DONE / 2;
-        int best_l = 0, dl = d_start;
-        xdrop_window30<0u>(s1tab_sa, s1_m10, s1_m9, rev2groups(ft), rev2groups(fq), fn, X, best_l, dl, nchunks);
-#pragma unroll 1
-        for (int b = 1; b < S1_LEFT_WINDOWS; b++) {
-            if (__all_sync(0xffffffffu, dl >= S1_DONE / 2)) break;
-            uint64_t wt = 0, wq = 0; uint32_t an = 0;
-            if (dl < S1_DONE / 2) {
-                const uint32_t ct = hi + SEED_SPAN - S1_WINDOW * b - 32, cq = hj + SEED_SPAN - S1_WINDOW * b - 32;
-                wt = window32(T.pk, ct); wq = window32(Q.pk, cq);
-                an = __brev(nwindow32(T.nm, ct) | nwindow32(Q.nm, cq)) & S1_WINDOW_MASK;
+            if (!__all_sync(0xffffffffu, dl >= S1_DONE / 2)) {
+                s1_later_window(T, Q, hi, hj, false, 2, dl, wt, wq, an);
+                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, wt, wq, an, X, best_l, dl, nchunks);
             }
-            xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, rev2groups(wt), rev2groups(wq), an, X, best_l, dl, nchunks);
+        } else {
+            // ---------------- phase B: one batch of up to 32 hits, one per lane
+            const uint32_t nb = min(pending, 32u);
+            live = (uint32_t)lane < nb;
+            const uint32_t h = consumed + (uint32_t)lane;
+            uint32_t e_last = head;
+            {
+                // Descriptor of every hit of the batch without a search: rc[head] <= consumed < rc[head + 1] (invariant of `head`) and
+                // every descriptor holds at least one hit, so the batch lies inside descriptors head .. head + 31. Lane i looks at
+                // descriptor head + i; the ones that START inside the batch (at offset 1..31) set a bit at their offset; the
+                // descriptor of the hit at offset l is head + (bits at or below l).
+                const uint32_t di = head + (uint32_t)lane;
+                const bool dv = (int32_t)(tail - di) > 0;
+                const uint32_t ci = dv ? rc[di & (SC_RING - 1)] : 0u;
+                const uint32_t first = ci - consumed;                   // wrapping; >= 1 for lane > 0
+                const uint32_t starts = __reduce_or_sync(0xffffffffu, (dv && lane > 0 && first < 32u) ? (1u << first) : 0u);
+                if (live) {
+                    const uint32_t lo = head + (uint32_t)__popc(starts & ((2u << lane) - 1u));
+                    e_last = lo;
+                    hi = pos[rb[lo & (SC_RING - 1)] + (h - rc[lo & (SC_RING - 1)])];
+                    hj = rj[lo & (SC_RING - 1)];
+                }
+            }
+            // Everything the batch needs that does not depend on the x-drop outcome: leader window (p - 1), first right window
+            // (p + 19) and first left window (p - 13). All three lie inside the 128 columns that start at the 64-column boundary
+            // below p - 13, so each sequence is fetched as ONE aligned block (32 bytes of packed bases, 16 of flags: four load
+            // instructions per sequence instead of twelve) and the windows are cut out of registers. After the bank fix of the
+            // extension table (xdrop_table.cuh) the scan is bound by the integer ALU pipe (ncu on C4: alu pipe 74 % busy, L1 data
+            // pipe 65 %, DRAM 11 %; profiles/r2_seed_scan_c4_v2_ncu_summary.txt); taking the pos[] and target gathers of the next
+            // batch off the critical path (a pipelined variant, measured) changed nothing and was dropped.
+            uint64_t lt = 0, lq = 0, rt = 0, rq = 0, ft = 0, fq = 0;
+            uint32_t ln = 1, rn = 0, fn = 0;
+            if (live) {
+                const SeqBlock bt = load_block(T.pk, T.nm, T.sm, hi - 13), bq = load_block(Q.pk, Q.nm, Q.sm, hj - 13);
+                uint32_t tfn, trn, tls, qfn, qrn, qls;
+                bt.windows(hi - 13, ft, lt, rt, tfn, trn, tls);
+                bq.windows(hj - 13, fq, lq, rq, qfn, qrn, qls);
+                ln = (tls | qls) & SEED_WINDOW_MASK19;
+                rn = (trn | qrn) & S1_WINDOW_MASK;
+                fn = __brev(tfn | qfn) & S1_WINDOW_MASK;
+                // spec D1: only run leaders are candidates
+                if (ln == 0 && seed_match(lt, lq, transition != 0)) live = false; else n_lead++;
+            }
+            // Right of the seed: window 0 of 30 columns. Left, from the last seed column downwards: windows 0 and 1, reversed so
+            // that the same forward-order table applies. The first window of either side comes out of the blocks above and runs
+            // without polling (some lane of 32 is practically always still open at its end; on the left its first 19 columns are
+            // the seed itself); left window 1 (needed by ~90 % of hits) is skipped when all lanes are done and polled inside.
+            if (live) { dr = S1_D0; dl = S1_D0; }
+            xdrop_window30<0u>(s1tab_sa, s1_m10, s1_m9, rt, rq, rn, X, best_r, dr, nchunks);
+            xdrop_window30<0u>(s1tab_sa, s1_m10, s1_m9, rev2groups(ft), rev2groups(fq), fn, X, best_l, dl, nchunks);
+            if (!__all_sync(0xffffffffu, dl >= S1_DONE / 2)) {
+                uint64_t wt, wq; uint32_t an;
+                s1_later_window(T, Q, hi, hj, false, 1, dl, wt, wq, an);
+                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, wt, wq, an, X, best_l, dl, nchunks);
+            }
+            // a hit still open on either side goes to the queue and is decided by a drain, also one whose best_r + best_l already
+            // reaches K: stage1_cells counts every chunk a hit is open in
+            const bool defer = live && (dr < S1_DONE / 2 || dl < S1_DONE / 2);
+            const uint32_t dmask = __ballot_sync(0xffffffffu, defer);
+            if (defer) {
+                dq[(dq_tail + (uint32_t)__popc(dmask & ((1u << lane) - 1u))) & (SC_DQ - 1)] =
+                    make_uint4(hi, hj, s1_pack(best_r, dr), s1_pack(best_l, dl));
+                live = false;
+            }
+            dq_tail += (uint32_t)__popc(dmask);
+            // retire the batch: descriptors that are fully consumed leave the ring
+            consumed += nb;
+            uint32_t e = __shfl_sync(0xffffffffu, e_last, (int)nb - 1);
+            const uint32_t next_cum = (e + 1 < tail) ? rc[(e + 1) & (SC_RING - 1)] : cum_tail;
+            head = ((int32_t)(next_cum - consumed) > 0) ? e : e + 1;
         }
-        const bool open_l = dl < S1_DONE / 2;
         n_cells += 3ull * nchunks;
         // dead iff both sides terminated inside their bounds with a total below K (spec D2: failed extensions leave no trace)
-        const bool survivor = live && (open_r || open_l || (best_r + best_l >= K));
-        const uint32_t smask = __ballot_sync(0xffffffffu, survivor);
-        if (smask) {
-            unsigned long long basev = 0;
-            if (lane == __ffs(smask) - 1) basev = atomicAdd(&counters[0], (unsigned long long)__popc(smask));
-            basev = __shfl_sync(0xffffffffu, basev, __ffs(smask) - 1);
-            if (survivor) {
-                const unsigned long long slot = basev + __popc(smask & ((1u << lane) - 1u));
-                if (slot < surv_cap) surv[slot] = ((uint64_t)(hi - hj + diag_bias) << 32) | hj;
-            }
-        }
-        // retire the batch: descriptors that are fully consumed leave the ring
-        consumed += nb;
-        uint32_t e = __shfl_sync(0xffffffffu, e_last, (int)nb - 1);
-        const uint32_t next_cum = (e + 1 < tail) ? rc[(e + 1) & (SC_RING - 1)] : cum_tail;
-        head = ((int32_t)(next_cum - consumed) > 0) ? e : e + 1;
+        append_survivors(live && (dr < S1_DONE / 2 || dl < S1_DONE / 2 || best_r + best_l >= K), hi, hj, diag_bias, lane, surv, surv_cap, counters);
         __syncwarp();
     }
     // statistics
