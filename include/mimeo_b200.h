@@ -261,6 +261,33 @@ MB2_API int mb2_format_gff(const int32_t* chrom, const int32_t* start, const int
                            int nnames, const char* source, const char* label, const char* prefix, uint64_t first_id, int nthreads,
                            mb2_text* out);
 
+/* ---- tandem-repeat mask of `mimeo map --maxtandem` -------------------------------------------------- */
+/* The reference runs Tandem Repeats Finder on every A-genome hit span; this build computes its own mask (DESIGN §2,
+ * T1-T4; not TRF): local self-alignment of the span within diagonals 1..maxperiod, +match / -mismatch (N never matches),
+ * -delta per indel; a position is masked iff it lies between the two aligned positions of a column of some such
+ * alignment scoring >= minscore. Defaults = mimeo's --tmatch 2 --tmismatch 7 --tdelta 7 --tminscore 50 --tmaxperiod 50. */
+typedef struct mb2_tandem_params {
+    int32_t match, mismatch, delta, minscore, maxperiod;
+} mb2_tandem_params;
+MB2_API void mb2_default_tandem_params(mb2_tandem_params* p);
+/* masked[k] = number of masked positions of span k = scaffold scaf[k] of g, bases [start[k], start[k] + len[k]) (0-based;
+ * len 0 allowed). HOST arrays. Identical spans are computed once. Parameters out of range (match < 1, mismatch or delta < 0,
+ * minscore < 1, maxperiod outside 1..256, minscore + mismatch > 65535) or a span outside its scaffold: MB2_ERR_INVALID_ARG. */
+MB2_API int mb2_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                            const mb2_tandem_params* p, uint64_t* masked);
+/* Test hook: mb2_tandem_mask that also returns the merged masked runs of every span (span-local, closed [start, end]):
+ * run r of span k is (start[r], end[r]) for off[k] <= r < off[k+1]. store_budget = bytes of device storage per launch
+ * (0 = default; small values force many launches). Arrays owned by the library; free with mb2_free_tandem_runs. */
+typedef struct mb2_tandem_runs {
+    uint64_t* off;       /* n + 1 entries */
+    int64_t* start;
+    int64_t* end;
+    uint64_t n;
+} mb2_tandem_runs;
+MB2_API int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                                 const mb2_tandem_params* p, uint64_t store_budget, uint64_t* masked, mb2_tandem_runs* runs);
+MB2_API void mb2_free_tandem_runs(mb2_tandem_runs* r);
+
 /* ---- device primitives exposed for parity tests ------------------------------------------- */
 /* Stable LSD radix sort of HOST arrays on bits [begin_bit, end_bit) (vals may be NULL). */
 MB2_API int mb2_test_sort_u32(uint32_t* keys, uint32_t* vals, uint64_t n, int begin_bit, int end_bit);

@@ -51,6 +51,14 @@ class Text(C.Structure):
     _fields_ = [('text', C.POINTER(C.c_char)), ('nbytes', C.c_uint64), ('nrows', C.c_uint64)]
 
 
+class TandemParams(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ('match', 'mismatch', 'delta', 'minscore', 'maxperiod')]
+
+
+class TandemRuns(C.Structure):
+    _fields_ = [('off', c_u64p), ('start', c_i64p), ('end', c_i64p), ('n', C.c_uint64)]
+
+
 class Segments(C.Structure):
     _fields_ = [('chrom', c_i32p), ('start', c_i32p), ('end', c_i32p), ('n', C.c_uint64), ('on_device', C.c_int)]
 
@@ -103,6 +111,11 @@ SIGNATURES = {
     'mb2_format_gff': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_char_p), C.c_int, C.c_char_p, C.c_char_p,
                                  C.c_char_p, C.c_uint64, C.c_int, C.POINTER(Text)]),
     'mb2_free_text': (None, [C.POINTER(Text)]),
+    'mb2_default_tandem_params': (None, [C.POINTER(TandemParams)]),
+    'mb2_tandem_mask': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(TandemParams), C.c_void_p]),
+    'mb2_test_tandem_mask': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(TandemParams), C.c_uint64,
+                                       C.c_void_p, C.POINTER(TandemRuns)]),
+    'mb2_free_tandem_runs': (None, [C.POINTER(TandemRuns)]),
     'mb2_test_sort_u32': (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int]),
     'mb2_test_sort_u64': (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int]),
     'mb2_test_sort_u32_pair': (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int]),

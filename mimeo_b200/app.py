@@ -1,4 +1,5 @@
-"""`mimeo <x|self|map>` dispatcher (host mirror of src/mimeo/app.py:21-63). `filter` (TRF) is out of scope."""
+"""`mimeo <x|self|map>` dispatcher (host mirror of src/mimeo/app.py:21-63). The tandem-repeat filter runs inside
+`mimeo map --maxtandem` (GPU mask, DESIGN §2 T1-T4); the separate `filter` subcommand is not provided."""
 import sys
 from importlib import import_module
 

@@ -519,6 +519,54 @@ int mb2_hits_dev_download(const mb2_hits_dev* h, mb2_hits* out) {
     });
 }
 
+// ------------------------------------------------------------------------------------------ tandem mask
+void mb2_default_tandem_params(mb2_tandem_params* p) {
+    if (!p) return;
+    TandemParams d;
+    p->match = d.match; p->mismatch = d.mismatch; p->delta = d.delta; p->minscore = d.minscore; p->maxperiod = d.maxperiod;
+}
+static TandemParams to_tandem(const mb2_tandem_params* p) {
+    TandemParams t;
+    if (p) { t.match = p->match; t.mismatch = p->mismatch; t.delta = p->delta; t.minscore = p->minscore; t.maxperiod = p->maxperiod; }
+    return t;
+}
+int mb2_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                    const mb2_tandem_params* p, uint64_t* masked) {
+    return guarded([&] {
+        MB2_REQUIRE(g && g->g, MB2_ERR_INVALID_ARG, "tandem_mask: null genome");
+        tandem_mask(*g->g, scaf, start, len, n, to_tandem(p), 0, masked, nullptr);
+    });
+}
+int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                         const mb2_tandem_params* p, uint64_t store_budget, uint64_t* masked, mb2_tandem_runs* runs) {
+    return guarded([&] {
+        MB2_REQUIRE(g && g->g && runs, MB2_ERR_INVALID_ARG, "test_tandem_mask: null argument");
+        std::memset(runs, 0, sizeof(*runs));
+        std::vector<std::vector<std::pair<int64_t, int64_t>>> iv;
+        tandem_mask(*g->g, scaf, start, len, n, to_tandem(p), (size_t)store_budget, masked, &iv);
+        size_t total = 0;
+        for (const auto& v : iv) total += v.size();
+        runs->off = (uint64_t*)malloc((n + 1) * sizeof(uint64_t));
+        runs->start = (int64_t*)malloc((total ? total : 1) * sizeof(int64_t));
+        runs->end = (int64_t*)malloc((total ? total : 1) * sizeof(int64_t));
+        MB2_REQUIRE(runs->off && runs->start && runs->end, MB2_ERR_INTERNAL, "test_tandem_mask: host allocation failed");
+        runs->n = n;
+        runs->off[0] = 0;
+        for (uint64_t k = 0; k < n; k++) {
+            for (size_t t = 0; t < iv[k].size(); t++) {
+                runs->start[runs->off[k] + t] = iv[k][t].first;
+                runs->end[runs->off[k] + t] = iv[k][t].second;
+            }
+            runs->off[k + 1] = runs->off[k] + iv[k].size();
+        }
+    });
+}
+void mb2_free_tandem_runs(mb2_tandem_runs* r) {
+    if (!r) return;
+    free(r->off); free(r->start); free(r->end);
+    std::memset(r, 0, sizeof(*r));
+}
+
 // ------------------------------------------------------------------------------------------ test hooks
 int mb2_test_sort_u32(uint32_t* keys, uint32_t* vals, uint64_t n, int begin_bit, int end_bit) {
     return guarded([&] { test_sort<uint32_t>(keys, vals, n, begin_bit, end_bit); });

@@ -131,6 +131,12 @@ uint64_t format_segment_gff(const int32_t* chrom, const int32_t* start, const in
                             int nnames, const char* source, const char* label, const char* prefix, uint64_t first_id, int nthreads,
                             std::string& out);
 
+// tandem.cu : the tandem-repeat mask of `mimeo map --maxtandem` (m per span; intervals: merged masked runs, span-local
+// and closed, for the test hook). store_budget: bytes of stored backward scores per launch, 0 = default.
+struct TandemParams { int match = 2, mismatch = 7, delta = 7, minscore = 50, maxperiod = 50; };
+void tandem_mask(const Genome& g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n, const TandemParams& p,
+                 size_t store_budget, uint64_t* masked, std::vector<std::vector<std::pair<int64_t, int64_t>>>* intervals);
+
 // counters layout (device, unsigned long long[16])
 enum { CNT_SURV = 0, CNT_SEED_HITS = 1, CNT_LEADERS = 2, CNT_S1_CELLS = 3, CNT_HSPS = 4, CNT_EXTENDED = 5, CNT_S2_CELLS = 6,
        CNT_GAPPED_CELLS = 7, CNT_ALNS = 8, CNT_ANCHORS = 9, CNT_ERR = 10, CNT_WORK = 11, CNT_N = 16 };

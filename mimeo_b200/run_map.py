@@ -1,5 +1,8 @@
-"""`mimeo map` (host mirror of src/mimeo/run_map.py). The TRF options are accepted but the tandem-repeat filter is a
-separate tool outside the hot path (SURVEY 2.1): requesting --maxtandem raises."""
+"""`mimeo map` (host mirror of src/mimeo/run_map.py). With --maxtandem, hits whose A-genome span is masked by more than
+that percentage are dropped after numbering (import_Align -> tandem filter -> GFF3, SURVEY 3.3), so the surviving rows
+keep their IDs. The mask is this project's own GPU statement (DESIGN §2, T1-T4), not Tandem Repeats Finder: --TRFpath,
+--tPM and --tPI are accepted and have no effect. --writeTRF (with --maxtandem) also writes the .tab lines of the surviving
+hits to `<outfile without .tab>_TRFfiltered.tab`."""
 import argparse
 import logging
 import os
@@ -7,10 +10,11 @@ import shutil
 import sys
 from typing import List
 
+from . import tandem
 from ._cli_common import add_loglevel, add_version
 from .logs import init_logging
 from .utils import chromlens, get_all_pairs, run_cmd, set_paths
-from .wrappers import import_Align, map_LZ_cmds, write_map_gff, writeGFFlines  # noqa: F401  (the pandas pair stays importable)
+from .wrappers import import_Align, map_LZ_cmds, map_gff_text, write_map_gff, writeGFFlines  # noqa: F401  (the pandas pair stays importable)
 
 
 def mainArgs() -> argparse.Namespace:
@@ -32,16 +36,16 @@ def mainArgs() -> argparse.Namespace:
     parser.add_argument('--minIdt', type=int, default=60, help='Minimum alignment identity to report.')
     parser.add_argument('--minLen', type=int, default=100, help='Minimum alignment length to report.')
     parser.add_argument('--hspthresh', type=int, default=3000, help='Set HSP min score threshold.')
-    parser.add_argument('--TRFpath', type=str, default='trf', help='Custom path to TRF executable if not in $PATH.')
-    parser.add_argument('--tmatch', type=int, default=2, help='TRF matching weight')
-    parser.add_argument('--tmismatch', type=int, default=7, help='TRF mismatching penalty')
-    parser.add_argument('--tdelta', type=int, default=7, help='TRF indel penalty')
-    parser.add_argument('--tPM', type=int, default=80, help='TRF match probability')
-    parser.add_argument('--tPI', type=int, default=10, help='TRF indel probability')
-    parser.add_argument('--tminscore', type=int, default=50, help='TRF minimum alignment score to report')
-    parser.add_argument('--tmaxperiod', type=int, default=50, help='TRF maximum period size to report')
-    parser.add_argument('--maxtandem', type=float, default=None, help='Max percentage of an A-genome alignment which may be masked by TRF.')
-    parser.add_argument('--writeTRF', action='store_true', default=False, help='If set write TRF filtered alignment file.')
+    parser.add_argument('--TRFpath', type=str, default='trf', help='Accepted for compatibility; the tandem repeat mask runs on the GPU.')
+    parser.add_argument('--tmatch', type=int, default=2, help='Tandem mask matching weight (>= 1)')
+    parser.add_argument('--tmismatch', type=int, default=7, help='Tandem mask mismatch penalty (>= 0)')
+    parser.add_argument('--tdelta', type=int, default=7, help='Tandem mask indel penalty (>= 0)')
+    parser.add_argument('--tPM', type=int, default=80, help='Accepted for compatibility; no effect (DESIGN T1).')
+    parser.add_argument('--tPI', type=int, default=10, help='Accepted for compatibility; no effect (DESIGN T1).')
+    parser.add_argument('--tminscore', type=int, default=50, help='Tandem mask minimum alignment score (>= 1)')
+    parser.add_argument('--tmaxperiod', type=int, default=50, help='Tandem mask maximum period (1..256)')
+    parser.add_argument('--maxtandem', type=float, default=None, help='Max percentage of an A-genome alignment which may be masked as tandem repeat.')
+    parser.add_argument('--writeTRF', action='store_true', default=False, help='With --maxtandem, also write the alignments that pass the filter.')
     add_loglevel(parser)
     return parser.parse_args()
 
@@ -50,8 +54,9 @@ def main() -> None:
     args = mainArgs()
     init_logging(loglevel=args.loglevel)
     logging.info('Starting genome mapping workflow.')
+    tparams = None
     if args.maxtandem:
-        raise RuntimeError('--maxtandem needs Tandem Repeats Finder, which is outside the GPU hot path of this build')
+        tparams = tandem.params(args.tmatch, args.tmismatch, args.tdelta, args.tminscore, args.tmaxperiod)
     adir_path, bdir_path, outdir, outtab, gffout, tempdir = set_paths(
         adir=args.adir, bdir=args.bdir, afasta=args.afasta, bfasta=args.bfasta, outdir=args.outdir, outtab=args.outfile,
         gffout=args.gffout, runtrf=args.maxtandem)
@@ -67,8 +72,16 @@ def main() -> None:
         logging.info('Running alignments...')
         run_cmd(cmds, verbose=args.verbose, keeptemp=args.keeptemp)
     # import_Align + writeGFFlines (still importable from .wrappers) in one native pass over the .tab file
-    write_map_gff(infile=outtab, gffout=gffout, chrlens=chrLens, prefix=args.prefix, minLen=args.minLen, minIdt=args.minIdt,
-                  ftype=args.label)
+    if tparams is None:
+        write_map_gff(infile=outtab, gffout=gffout, chrlens=chrLens, prefix=args.prefix, minLen=args.minLen, minIdt=args.minIdt,
+                      ftype=args.label)
+    else:
+        n, body = map_gff_text(outtab, args.prefix, args.minLen, args.minIdt, args.label)
+        if n == 0:
+            logging.warning('No alignments found in %s' % outtab)
+            sys.exit(1)
+        tandem.write_filtered_map(outtab, body, gffout, chrLens, adir_path, args.maxtandem, tparams,
+                                  tandem.trf_path(outtab) if args.writeTRF else None)
     if tempdir and os.path.isdir(tempdir) and not args.keeptemp:
         shutil.rmtree(tempdir)
     logging.info('Finished!')
