@@ -135,6 +135,22 @@ MB2_API void mb2_free_hsps(mb2_hsps* h);
  * [0] survivors [1] seed hits [2] run leaders [3] stage-1 cells [4] HSPs [5] extensions [6] stage-2 cells. */
 MB2_API int mb2_test_hsps(const mb2_genome* T, const mb2_genome* Q, const mb2_align_params* p, mb2_hsps* out, uint64_t* stats);
 
+/* Test hook: stage (a) only. The seed hits of T x Q that the bounded first-stage x-drop could not rule out (one scan of the
+ * whole query), as PADDED positions: the seed of survivor k starts at t_pos[k] in T and q_pos[k] in Q, in the order the scan
+ * wrote them. t_off / q_off: padded start of every scaffold of T / Q. counters: [0] survivors [1] seed hits [2] run leaders
+ * [3] stage-1 cells. init_cap = initial survivor capacity (0 = default); a smaller value forces the overflow and rescan.
+ * HOST arrays owned by the library; free with mb2_free_seed_survivors. */
+typedef struct mb2_seed_survivors {
+    uint32_t *t_pos, *q_pos;
+    uint64_t n;
+    uint32_t *t_off, *q_off;
+    int32_t t_nscaf, q_nscaf;
+    uint64_t counters[4];
+} mb2_seed_survivors;
+MB2_API int mb2_test_seed_scan(const mb2_genome* T, const mb2_genome* Q, const mb2_align_params* p, uint64_t init_cap,
+                               mb2_seed_survivors* out);
+MB2_API void mb2_free_seed_survivors(mb2_seed_survivors* s);
+
 /* ---- (a)+(b)+(b')+(c): the whole LASTZ stage ------------------------------------------------ */
 /* One row per gapped alignment, i.e. per line of LASTZ's --format=general output before mimeo's
  * awk filters (wrappers.py:1044-1056). start1/end1/start2/end2 are what LASTZ prints: origin-one,

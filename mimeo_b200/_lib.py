@@ -27,6 +27,11 @@ class Hsps(C.Structure):
     _fields_ = [('tile', c_u32p), ('s1', c_i32p), ('s2', c_i32p), ('len', c_i32p), ('score', c_i32p), ('n', C.c_uint64)]
 
 
+class SeedSurvivors(C.Structure):
+    _fields_ = [('t_pos', c_u32p), ('q_pos', c_u32p), ('n', C.c_uint64), ('t_off', c_u32p), ('q_off', c_u32p),
+                ('t_nscaf', C.c_int32), ('q_nscaf', C.c_int32), ('counters', C.c_uint64 * 4)]
+
+
 class Hits(C.Structure):
     _fields_ = [(n, c_i32p) for n in ('t_id', 'q_id', 'strand', 'start1', 'end1', 'start2', 'end2', 'score', 'nmatch', 'ncols')] + \
                [('n', C.c_uint64), ('stats', C.c_uint64 * 16)]
@@ -90,6 +95,8 @@ SIGNATURES = {
     'mb2_default_align_params': (None, [C.POINTER(AlignParams)]),
     'mb2_free_hsps': (None, [C.POINTER(Hsps)]),
     'mb2_test_hsps': (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(AlignParams), C.POINTER(Hsps), C.c_void_p]),
+    'mb2_test_seed_scan': (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(AlignParams), C.c_uint64, C.POINTER(SeedSurvivors)]),
+    'mb2_free_seed_survivors': (None, [C.POINTER(SeedSurvivors)]),
     'mb2_align': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(AlignParams), C.c_int, C.c_void_p, C.POINTER(Hits)]),
     'mb2_free_hits': (None, [C.POINTER(Hits)]),
     'mb2_align_dev': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(AlignParams), C.c_int, C.c_void_p, C.POINTER(C.c_void_p)]),

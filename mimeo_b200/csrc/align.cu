@@ -99,6 +99,28 @@ void align_hsps(const Genome& T, const Genome& Q, const AlignParams& p, HspSet& 
     }
 }
 
+// Test hook (stage a only): the survivors of one scan of the whole query, through scan_chunk (and so through its overflow and
+// rescan when init_cap is too small). The query range is that of align_strand's chunks: first to last base.
+void scan_survivors(const Genome& T, const Genome& Q, const AlignParams& p, uint64_t init_cap, std::vector<uint64_t>& surv,
+                    unsigned long long* h_counters) {
+    Ctx& cx = ctx();
+    MB2_REQUIRE(T.G + Q.G < 0xffffffffull, -3, "scan: target + query exceed 2^32 padded positions");
+    DevBuf<unsigned long long> counters(CNT_N);
+    SeedTable tab;
+    build_seed_table(T, 0, (uint32_t)T.G, tab);
+    uint64_t cap = init_cap ? init_cap : std::max<uint64_t>(1u << 20, (T.nbases + Q.nbases) / 2);
+    DevBuf<uint64_t> s0;
+    unsigned long long nsurv = 0, acc[CNT_N] = {0};
+    uint32_t q_lo, q_hi;
+    chunk_range(Q, QChunk{0, Q.nscaf}, q_lo, q_hi);
+    const bool ok = scan_chunk(T, Q, tab, q_lo, q_hi, p, s0, cap, counters.get(), nsurv, acc);
+    MB2_REQUIRE(ok, -3, "scan: too many surviving seed hits for one pass");
+    surv.resize(nsurv);
+    if (nsurv) MB2_CUDA(cudaMemcpyAsync(surv.data(), s0.get(), nsurv * sizeof(uint64_t), cudaMemcpyDeviceToHost, cx.stream));
+    MB2_CUDA(cudaStreamSynchronize(cx.stream));
+    for (int k = 0; k < 4; k++) h_counters[k] = acc[k];
+}
+
 // Full pipeline for one strand-oriented query genome; the alignments of every query chunk are appended to the device hit
 // table `out` in LASTZ's output columns.
 void align_strand(const Genome& T, const Genome& Q, const AlignParams& p, const int32_t* h_same_q, DevHits& out, int nq, int strands,

@@ -7,6 +7,7 @@
 #include "primitives.cuh"
 #include "internal.cuh"
 #include "seq.cuh"
+#include "xdrop_table.cuh"
 #include "mimeo_b200.h"
 
 namespace mb2 {
@@ -341,8 +342,17 @@ static AlignParams to_params(const mb2_align_params* p) {
         a.hspthresh = p->hspthresh; a.xdrop = p->xdrop; a.ydrop = p->ydrop; a.gap_open = p->gap_open; a.gap_extend = p->gap_extend;
         a.gappedthresh = p->gappedthresh; a.entropy = p->entropy; a.chain = p->chain; a.gapped = p->gapped; a.transition = p->transition;
     }
-    MB2_REQUIRE(a.xdrop > 0 && a.ydrop > 0 && a.gap_open >= 0 && a.gap_extend > 0 && a.hspthresh > 0, MB2_ERR_INVALID_ARG,
-                "align params out of range");
+    MB2_REQUIRE(a.hspthresh > 0, MB2_ERR_INVALID_ARG, "align params: hspthresh must be positive");
+    MB2_REQUIRE(a.xdrop >= XT_MIN_XDROP, MB2_ERR_INVALID_ARG,
+                "align params: x-drop below 251 is not supported (the three-column extension table needs x-drop > 250)");
+    MB2_REQUIRE(a.xdrop <= GF_MAX_XDROP, MB2_ERR_INVALID_ARG,
+                "align params: x-drop of 6400 or more is not supported (a gap-free extension could cross the 64-column pad "
+                "between two scaffolds, which loses only 6400)");
+    MB2_REQUIRE(a.ydrop >= YDROP_MIN && a.ydrop <= YDROP_MAX && a.gap_open >= 0 && a.gap_open <= GAP_OPEN_MAX &&
+                    a.gap_extend >= GAP_EXTEND_MIN && a.gap_extend <= GAP_EXTEND_MAX,
+                MB2_ERR_INVALID_ARG,
+                "align params: y-drop must lie in 1000..20000, gap open in 0..2000 and gap extend in 10..60 "
+                "(the range of the 16-bit gapped extension kernel)");
     return a;
 }
 
@@ -375,6 +385,41 @@ int mb2_test_hsps(const mb2_genome* T, const mb2_genome* Q, const mb2_align_para
         out->len = to_host(h.len, h.n); out->score = to_host(h.score, h.n);
         MB2_CUDA(cudaStreamSynchronize(g_ctx.stream));
         if (stats) for (int k = 0; k < CNT_N; k++) stats[k] = cnt[k];
+    });
+}
+
+void mb2_free_seed_survivors(mb2_seed_survivors* s) {
+    if (!s) return;
+    free(s->t_pos); free(s->q_pos); free(s->t_off); free(s->q_off);
+    std::memset(s, 0, sizeof(*s));
+}
+
+int mb2_test_seed_scan(const mb2_genome* T, const mb2_genome* Q, const mb2_align_params* p, uint64_t init_cap,
+                       mb2_seed_survivors* out) {
+    return guarded([&] {
+        ensure_init();
+        MB2_REQUIRE(T && Q && T->g && Q->g && out, MB2_ERR_INVALID_ARG, "test_seed_scan: null argument");
+        std::memset(out, 0, sizeof(*out));
+        std::vector<uint64_t> surv;
+        unsigned long long cnt[4];
+        scan_survivors(*T->g, *Q->g, to_params(p), init_cap, surv, cnt);
+        const size_t n = surv.size();
+        const uint32_t qG = (uint32_t)Q->g->G;
+        out->t_pos = (uint32_t*)malloc((n ? n : 1) * sizeof(uint32_t));
+        out->q_pos = (uint32_t*)malloc((n ? n : 1) * sizeof(uint32_t));
+        out->t_off = (uint32_t*)malloc(T->g->nscaf * sizeof(uint32_t));
+        out->q_off = (uint32_t*)malloc(Q->g->nscaf * sizeof(uint32_t));
+        MB2_REQUIRE(out->t_pos && out->q_pos && out->t_off && out->q_off, MB2_ERR_INTERNAL, "test_seed_scan: host allocation failed");
+        for (size_t k = 0; k < n; k++) {
+            const uint32_t qj = (uint32_t)surv[k];
+            out->q_pos[k] = qj;
+            out->t_pos[k] = (uint32_t)(surv[k] >> 32) - qG + qj;      // survivors hold (diagonal + Q.G, query position)
+        }
+        out->n = n;
+        std::memcpy(out->t_off, T->g->off.data(), T->g->nscaf * sizeof(uint32_t));
+        std::memcpy(out->q_off, Q->g->off.data(), Q->g->nscaf * sizeof(uint32_t));
+        out->t_nscaf = T->g->nscaf; out->q_nscaf = Q->g->nscaf;
+        for (int k = 0; k < 4; k++) out->counters[k] = cnt[k];
     });
 }
 

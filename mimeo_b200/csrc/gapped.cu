@@ -245,8 +245,8 @@ struct GpWork {
     uint8_t* status;                 // [2 * nmember]: slot * 2 + direction (0 forward, 1 backward)
     int32_t *e_score, *e_di, *e_dj, *e_nm, *e_nc;   // [2 * nmember] one-sided extension results
     uint32_t* stamp;                 // per cluster: last round that scheduled one of its members
-    uint32_t *items_narrow, *items_wide;   // work lists of this round: slot * 2 + direction
-    uint32_t* counts;                // {narrow, wide}
+    uint32_t *items_narrow, *items_wide, *items_full;   // work lists of this round: slot * 2 + direction
+    uint32_t* counts;                // {narrow, wide, full rows (band wider than the wide kernel)}
 };
 
 constexpr int SEL_PEND = 64;         // pending (computed, not yet accepted) boxes a warp remembers while scheduling
@@ -389,6 +389,7 @@ gp_forward_kernel(GenomeView T, GenomeView Q, GpWork W, const uint32_t* __restri
             atomicAdd(&counters[CNT_GAPPED_CELLS], (unsigned long long)r.cells);
             if (r.status == yw::ST_NOMEM) { W.status[item] = GX_NONE; atomicAdd(&counters[CNT_WORK], 1ull); }       // scheduled again next round
             else if (r.status == yw::ST_WIDE) W.status[item] = GX_NEED_WIDE;
+            else if (r.status == yw::ST_BAND) W.items_full[atomicAdd(&W.counts[2], 1u)] = item;     // gp_full_kernel, same round
             else if (r.status != yw::ST_OK) atomicAdd(&counters[CNT_ERR], 1ull);
         }
     }
@@ -414,6 +415,39 @@ gp_walk_kernel(GenomeView T, GenomeView Q, GpWork W, const uint32_t* __restrict_
         const yw::ExtResult r = res[item];
         W.e_score[item] = r.score; W.e_di[item] = r.di; W.e_dj[item] = r.dj; W.e_nm[item] = r.nmatch; W.e_nc[item] = r.ncols;
         if (r.status != yw::ST_OK) atomicAdd(&counters[CNT_ERR], 1ull);
+    }
+}
+
+// the round's ST_BAND items (alive band wider than the wide kernel's 2048 diagonals): the spec's recurrence on full rows,
+// one warp per item (yw::ydrop_full_warp); `rows` holds 3 * cap cells per warp
+constexpr int GP_FULL_WARPS = 32;
+constexpr int64_t GP_FULL_CAP = 1 << 16;
+__global__ void __launch_bounds__(32)
+gp_full_kernel(GenomeView T, GenomeView Q, GpWork W, uint32_t* __restrict__ next_item, const uint32_t* __restrict__ tile, yw::Params prm,
+               yw::FullCell* __restrict__ rows, yw::ExtResult* __restrict__ res, unsigned long long* __restrict__ counters) {
+    const int lane = threadIdx.x;
+    const uint32_t nitems = W.counts[2];
+    yw::FullCell* my = rows + (size_t)blockIdx.x * 3 * GP_FULL_CAP;
+    for (;;) {
+        uint32_t w = 0;
+        if (lane == 0) w = atomicAdd(next_item, 1u);
+        w = __shfl_sync(0xffffffffu, w, 0);
+        if (w >= nitems) break;
+        const uint32_t item = W.items_full[w];
+        const uint32_t x = item >> 1, dir = item & 1u;
+        const uint32_t tl = tile[W.order[x]];
+        const uint32_t tsc = tl / (uint32_t)Q.nscaf, qsc = tl % (uint32_t)Q.nscaf;
+        const int a1 = W.a1[x], a2 = W.a2[x];
+        const int64_t tn = dir == 0 ? (int64_t)T.len[tsc] - a1 : a1, qn = dir == 0 ? (int64_t)Q.len[qsc] - a2 : a2;
+        yw::ydrop_full_warp(T.codes, Q.codes, (int64_t)T.off[tsc] + a1, (int64_t)Q.off[qsc] + a2, dir == 0 ? +1 : -1, tn, qn, prm, my,
+                            GP_FULL_CAP, &res[item]);
+        __syncwarp();
+        if (lane == 0) {
+            const yw::ExtResult r = res[item];
+            atomicAdd(&counters[CNT_GAPPED_CELLS], (unsigned long long)r.cells);
+            W.e_score[item] = r.score; W.e_di[item] = r.di; W.e_dj[item] = r.dj; W.e_nm[item] = r.nmatch; W.e_nc[item] = r.ncols;
+            if (r.status != yw::ST_OK) atomicAdd(&counters[CNT_ERR], 1ull);
+        }
     }
 }
 
@@ -575,7 +609,7 @@ void gapped_extend(const Genome& T, const Genome& Q, const HspSet& h, const DevB
             // anchors, per-slot state
             DevBuf<int32_t> a1(nm), a2(nm), e_score(2 * (size_t)nm), e_di(2 * (size_t)nm), e_dj(2 * (size_t)nm), e_nm(2 * (size_t)nm), e_nc(2 * (size_t)nm);
             DevBuf<uint8_t> status(2 * (size_t)nm);
-            DevBuf<uint32_t> items_n(2 * (size_t)nm), items_w(2 * (size_t)nm), counts(2), resume(h_nseg), nkept(h_nseg);
+            DevBuf<uint32_t> items_n(2 * (size_t)nm), items_w(2 * (size_t)nm), items_f(2 * (size_t)nm), counts(3), resume(h_nseg), nkept(h_nseg);
             MB2_CUDA(cudaMemsetAsync(status.get(), 0, 2 * (size_t)nm, cx.stream));
             MB2_CUDA(cudaMemsetAsync(resume.get(), 0, (size_t)h_nseg * sizeof(uint32_t), cx.stream));
             MB2_CUDA(cudaMemsetAsync(nkept.get(), 0, (size_t)h_nseg * sizeof(uint32_t), cx.stream));
@@ -592,11 +626,12 @@ void gapped_extend(const Genome& T, const Genome& Q, const HspSet& h, const DevB
             GpWork W;
             W.order = order; W.a1 = a1.get(); W.a2 = a2.get(); W.cluster_of = cluster_of.get(); W.status = status.get();
             W.e_score = e_score.get(); W.e_di = e_di.get(); W.e_dj = e_dj.get(); W.e_nm = e_nm.get(); W.e_nc = e_nc.get();
-            W.stamp = stamp.get(); W.items_narrow = items_n.get(); W.items_wide = items_w.get(); W.counts = counts.get();
+            W.stamp = stamp.get(); W.items_narrow = items_n.get(); W.items_wide = items_w.get(); W.items_full = items_f.get(); W.counts = counts.get();
             static const bool dbg = getenv("MB2_GP_DEBUG") != nullptr;
             cudaEvent_t ev0 = nullptr, ev1 = nullptr;
             if (dbg) { cudaEventCreate(&ev0); cudaEventCreate(&ev1); }
-            MB2_REQUIRE(p.ydrop >= 1000 && p.ydrop <= 20000 && p.gap_open >= 0 && p.gap_open <= 2000 && p.gap_extend >= 10 && p.gap_extend <= 60,
+            MB2_REQUIRE(p.ydrop >= YDROP_MIN && p.ydrop <= YDROP_MAX && p.gap_open >= 0 && p.gap_open <= GAP_OPEN_MAX &&
+                        p.gap_extend >= GAP_EXTEND_MIN && p.gap_extend <= GAP_EXTEND_MAX,
                         -2, "gapped stage: y-drop / gap penalties outside the range the 16-bit extension kernel supports");
             const yw::Params prm{p.gap_open, p.gap_extend, p.ydrop};
             const int nslots = cx.sm_count * GP_WARPS_PER_SM;
@@ -604,11 +639,12 @@ void gapped_extend(const Genome& T, const Genome& Q, const HspSet& h, const DevB
             yw::Pool pool_wide = pool;
             pool_wide.priv = 0;              // the wide-band kernel runs in the same round: its traces go to the shared part only
             DevBuf<yw::ExtResult> res(2 * (size_t)nm);
-            DevBuf<uint32_t> next_item(2);
+            DevBuf<uint32_t> next_item(3);
+            DevBuf<yw::FullCell> full_rows;  // allocated by the first round that has an item for gp_full_kernel
             unsigned long long h_nomem_before = 0;
             uint32_t prev_sched = 0, conc = (uint32_t)nslots;      // items launched last round; CTAs (= concurrent extensions) allowed
             for (uint32_t round = 1;; round++) {
-                MB2_CUDA(cudaMemsetAsync(counts.get(), 0, 2 * sizeof(uint32_t), cx.stream));
+                MB2_CUDA(cudaMemsetAsync(counts.get(), 0, 3 * sizeof(uint32_t), cx.stream));
                 launch(gp_select_kernel, cdiv((size_t)h_nseg * 32, 128), 128, 0, W, h.tile.get(), nm, seg_start.get(), h_nseg, resume.get(), nkept.get(),
                        round, p.gappedthresh, r_s1.get(), r_e1.get(), r_s2.get(), r_e2.get(), r_score.get(), r_nm.get(), r_nc.get(), r_tile.get(),
                        keep.get(), counters);
@@ -636,7 +672,7 @@ void gapped_extend(const Genome& T, const Genome& Q, const HspSet& h, const DevB
                 prev_sched = h_counts[0] + h_counts[1];
                 h_nomem_before = h_nomem;
                 MB2_CUDA(cudaMemsetAsync(pool.next, 0, yw::NSUB * sizeof(uint32_t), cx.stream));      // previous round's traces are consumed
-                MB2_CUDA(cudaMemsetAsync(next_item.get(), 0, 2 * sizeof(uint32_t), cx.stream));
+                MB2_CUDA(cudaMemsetAsync(next_item.get(), 0, 3 * sizeof(uint32_t), cx.stream));
                 static const uint32_t lay_narrow = layout_mask("MB2_GP_LAYOUTS", "16,24,32"), lay_wide = lay_narrow | (1u << 12) | (1u << 16);
                 static const bool sort_items = !getenv("MB2_GP_NOSORT");
                 static const int occ = getenv("MB2_GP_OCC") ? atoi(getenv("MB2_GP_OCC")) : 16;
@@ -668,6 +704,17 @@ void gapped_extend(const Genome& T, const Genome& Q, const HspSet& h, const DevB
                     if (h_counts[0]) launch(gp_walk_kernel, cdiv(h_counts[0], 4), 128, 0, tv, qv, W, it_n, h_counts[0], h.tile.get(), prm, pool, res.get(), counters);
                     if (h_counts[1]) launch(gp_walk_kernel, cdiv(h_counts[1], 4), 128, 0, tv, qv, W, (const uint32_t*)items_w.get(), h_counts[1], h.tile.get(), prm, pool, res.get(), counters);
                 }
+                if (h_counts[1]) {                 // only the wide kernel hands out ST_BAND items; rounds with wide items are rare
+                    uint32_t h_full = 0;
+                    MB2_CUDA(cudaMemcpyAsync(&h_full, counts.get() + 2, sizeof(uint32_t), cudaMemcpyDeviceToHost, cx.stream));
+                    MB2_CUDA(cudaStreamSynchronize(cx.stream));
+                    if (h_full) {
+                        ProfScope pfull("gp_full");
+                        if (!full_rows.get()) full_rows.alloc((size_t)GP_FULL_WARPS * 3 * GP_FULL_CAP);
+                        launch(gp_full_kernel, std::min<uint32_t>(h_full, GP_FULL_WARPS), 32, 0, tv, qv, W, next_item.get() + 2, h.tile.get(), prm,
+                               full_rows.get(), res.get(), counters);
+                    }
+                }
                 if (dbg) cudaEventRecord(ev1, cx.stream);
             }
             if (dbg) { cudaEventDestroy(ev0); cudaEventDestroy(ev1); }
@@ -678,7 +725,7 @@ void gapped_extend(const Genome& T, const Genome& Q, const HspSet& h, const DevB
     MB2_CUDA(cudaMemcpyAsync(&h_nout, d_nout.get(), sizeof(uint32_t), cudaMemcpyDeviceToHost, cx.stream));
     MB2_CUDA(cudaMemcpyAsync(&h_err, counters + CNT_ERR, sizeof(h_err), cudaMemcpyDeviceToHost, cx.stream));
     MB2_CUDA(cudaStreamSynchronize(cx.stream));
-    MB2_REQUIRE(h_err == 0, -5, "gapped stage: an extension failed (band wider than 1900 diagonals, or an inconsistent trace)");
+    MB2_REQUIRE(h_err == 0, -5, "gapped stage: an extension failed (an anti-diagonal wider than 65536 cells, or an inconsistent trace)");
     out.n = h_nout;
     if (h_nout == 0) return;
     out.tile.alloc(h_nout); out.s1.alloc(h_nout); out.e1.alloc(h_nout); out.s2.alloc(h_nout); out.e2.alloc(h_nout);

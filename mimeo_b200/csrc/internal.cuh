@@ -29,6 +29,8 @@ struct AlignParams {   // LASTZ defaults for mimeo's command line (SURVEY 9.1)
     int hspthresh = 3000, xdrop = 910, ydrop = 9400, gap_open = 400, gap_extend = 30, gappedthresh = 3000;
     int entropy = 1, chain = 1, gapped = 1, transition = 1;
 };
+// y-drop and gap penalties the 16-bit gapped extension kernel supports (ydrop_warp.cuh)
+constexpr int YDROP_MIN = 1000, YDROP_MAX = 20000, GAP_OPEN_MAX = 2000, GAP_EXTEND_MIN = 10, GAP_EXTEND_MAX = 60;
 
 // genome.cu
 Genome* genome_from_ascii(const uint8_t* const* seqs, const uint64_t* lens, int n);
@@ -86,6 +88,10 @@ void hits_coverage(const DevHits& h, int which, const int64_t* h_sizes, int nchr
 
 // align.cu
 void align_hsps(const Genome& T, const Genome& Q, const AlignParams& p, HspSet& hsps, unsigned long long* h_counters);
+// test hook (stage a only): survivors of one scan of the whole query as (diagonal + Q.G) << 32 | query position, in scan
+// order; init_cap = initial survivor capacity (0 = default); h_counters[0..3] = survivors, seed hits, leaders, stage-1 cells
+void scan_survivors(const Genome& T, const Genome& Q, const AlignParams& p, uint64_t init_cap, std::vector<uint64_t>& surv,
+                    unsigned long long* h_counters);
 
 // whole pipeline for one (strand-oriented) query genome; rows are appended to `out` (nq, strands: see DevHits::append)
 void align_strand(const Genome& T, const Genome& Q, const AlignParams& p, const int32_t* h_same_q, DevHits& out, int nq, int strands,

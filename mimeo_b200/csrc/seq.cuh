@@ -4,7 +4,8 @@
 // and is surrounded by at least 64 pad bases (2048 at both ends of the genome) that are flagged non-ACGT, so that
 //   * a 19-mer seed window can never span two scaffolds,
 //   * gap-free x-drop extension needs no bounds checks: a pad column scores -100 like any
-//     non-ACGT character, so ten of them end the extension without changing its maximum,
+//     non-ACGT character, so the 64 columns of the narrowest pad lose 6400 and end every extension whose
+//     x-drop is below that (GF_MAX_XDROP) without changing its maximum,
 //   * unaligned 64-bit window reads one word past a scaffold are always in bounds.
 // Storage: pk  = 2 bits/base, 32 bases per uint64 word, base p in bits [2(p%32), 2(p%32)+1];
 //          nm  = 1 bit/base, 32 bases per uint32 word, 1 = not A/C/G/T (N, IUPAC, pad): scores -100 in every extension;
@@ -55,6 +56,8 @@ inline GenomeView view(const Genome& g) { return GenomeView{g.pk.get(), g.nm.get
 // HOXD70 as LASTZ's default, row = target base, col = query base (index t*4+q)
 static __constant__ int c_sub[16] = {91, -114, -31, -123, -114, 100, -125, -31, -31, -125, 100, -114, -123, -31, -114, 91};
 constexpr int SCORE_N = -100;
+// largest x-drop a gap-free extension may use: with 6400 or more it could walk through a 64-column pad into the next scaffold
+constexpr int GF_MAX_XDROP = -SCORE_N * (int)GENOME_PAD - 1;
 
 __device__ __forceinline__ uint32_t base_at(const uint64_t* __restrict__ pk, uint32_t p) {
     return (uint32_t)(pk[p >> 5] >> ((p & 31) * 2)) & 3u;

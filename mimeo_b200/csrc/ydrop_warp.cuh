@@ -57,7 +57,8 @@ constexpr int NSUB = 32;                     // sub-pools of the chunk allocator
 // scaffold (pad): a cell that would consume a pad base does not exist
 constexpr uint32_t CODE_N = 8, CODE_END = 12;
 
-enum : int { ST_OK = 0, ST_NOMEM = 1, ST_WIDE = 2, ST_FAIL = 3 };
+// ST_BAND: the alive band outgrew the widest layout (64 x 32 diagonals); the caller reruns the item with ydrop_full_warp
+enum : int { ST_OK = 0, ST_NOMEM = 1, ST_WIDE = 2, ST_FAIL = 3, ST_BAND = 4 };
 
 struct Params {
     int O, E, Y;          // gap open, gap extend, y-drop
@@ -602,7 +603,7 @@ YW_DEV void ydrop_forward_warp(const uint8_t* tcodes, const uint8_t* qcodes, int
         if (c.ahi < c.alo) break;                      // nothing alive (the dead-step test normally catches this first)
         const int need = c.ahi - c.alo + 1;
         int ns = pick_layout(c.lay_mask, need, 0, max_S);
-        if (ns == 0) { c.status = max_S >= 64 ? ST_FAIL : ST_WIDE; break; }    // ST_WIDE: the caller reruns the item with the wide kernel
+        if (ns == 0) { c.status = max_S >= 64 ? ST_BAND : ST_WIDE; break; }    // the caller reruns the item: wide kernel, then full rows
         const int slack = (32 * ns - need) / 2;
         c.S = ns;
         c.rbase = (c.alo - slack) & ~1;
@@ -801,6 +802,107 @@ YW_DEV void ydrop_walk_warp(const uint8_t* tcodes, const uint8_t* qcodes, int64_
     if (lane == 0) {
         res->di = di; res->dj = dj; res->nmatch = nm; res->ncols = nc;
         if (fail) res->status = ST_FAIL;
+    }
+}
+
+
+// ------------------------------------------------------------------------------------------ full-row fallback
+// The extensions whose band outgrows the widest layout (ST_BAND; e.g. y-drop 20000 with cheap gaps from an anchor inside a
+// repeat pair: the alive cells of one anti-diagonal then span more than 2048 diagonals). The spec's recurrence (the oracle's
+// ydrop_extend, D4) evaluated literally in 32-bit scores: every cell between the alive ranges of the two previous
+// anti-diagonals, three rows of FullCell in `rows` (3 * cap cells), (nmatch, ncols) carried along each state instead of a
+// trace. One warp, lane l takes cells clo + l, clo + l + 32, ...; slow, but only the rare ST_BAND items take it.
+// tn / qn = bases available from the anchor in the extension direction. Fills score, di, dj, nmatch, ncols, cells; status =
+// ST_OK, or ST_FAIL if an anti-diagonal needs more than cap cells.
+struct FullCell { int32_t h, d, i, hm, hc, dm, dc, im, ic; };
+constexpr int FULL_NEG = INT32_MIN / 4;
+
+YW_DEV int full_sub(uint32_t a, uint32_t b) {
+    if (a >= CODE_N || b >= CODE_N) return -100;
+    const int tab[16] = {91, -114, -31, -123, -114, 100, -125, -31, -31, -125, 100, -114, -123, -31, -114, 91};
+    return tab[((a & 3u) << 2) | (b & 3u)];
+}
+
+YW_DEV void ydrop_full_warp(const uint8_t* __restrict__ tcodes, const uint8_t* __restrict__ qcodes, int64_t ta, int64_t qa, int dir,
+                            int64_t tn, int64_t qn, const Params& p, FullCell* rows, int64_t cap, ExtResult* res) {
+    const int lane = lane_id();
+    FullCell *p2 = rows, *p1 = rows + cap, *cur = rows + 2 * cap;
+    int64_t b2 = 0, lo2 = 0, hi2 = -1, b1 = 0, lo1 = 0, hi1 = 0;   // row base (index of slot 0), alive range; k-1 = anti-diagonal 0
+    if (lane == 0) { FullCell z = {0, FULL_NEG, FULL_NEG, 0, 0, 0, 0, 0, 0}; p1[0] = z; }
+    syncwarp();
+    int best = 0, r_score = 0, r_di = 0, r_dj = 0, r_nm = 0, r_nc = 0, status = ST_OK;
+    uint64_t cells = 0;
+    for (int64_t k = 1; k <= tn + qn; k++) {
+        int64_t clo = INT64_MAX, chi = INT64_MIN;
+        if (hi1 >= lo1) { clo = lo1; chi = hi1 + 1; }
+        if (hi2 >= lo2) { if (lo2 + 1 < clo) clo = lo2 + 1; if (hi2 + 1 > chi) chi = hi2 + 1; }
+        if (clo == INT64_MAX) break;
+        if (clo < 0) clo = 0;
+        if (clo < k - qn) clo = k - qn;
+        if (chi > k) chi = k;
+        if (chi > tn) chi = tn;
+        int64_t nlo = INT64_MAX, nhi = INT64_MIN;
+        int amax = FULL_NEG;
+        if (chi >= clo) {
+            if (chi - clo + 1 > cap) { status = ST_FAIL; break; }
+            const int thr = best - p.Y;
+            for (int64_t i = clo + lane; i <= chi; i += 32) {
+                const int64_t j = k - i;
+                FullCell c = {FULL_NEG, FULL_NEG, FULL_NEG, 0, 0, 0, 0, 0, 0};
+                if (i - 1 >= lo1 && i - 1 <= hi1) {                       // up: (i-1, j) on k-1
+                    const FullCell u = p1[i - 1 - b1];
+                    if (u.h > FULL_NEG) {
+                        const int op = u.h - p.O - p.E, ex = u.d > FULL_NEG ? u.d - p.E : FULL_NEG;
+                        if (op >= ex) { c.d = op; c.dm = u.hm; c.dc = u.hc; } else { c.d = ex; c.dm = u.dm; c.dc = u.dc; }
+                    }
+                }
+                if (i >= lo1 && i <= hi1) {                               // left: (i, j-1) on k-1
+                    const FullCell l = p1[i - b1];
+                    if (l.h > FULL_NEG) {
+                        const int op = l.h - p.O - p.E, ex = l.i > FULL_NEG ? l.i - p.E : FULL_NEG;
+                        if (op >= ex) { c.i = op; c.im = l.hm; c.ic = l.hc; } else { c.i = ex; c.im = l.im; c.ic = l.ic; }
+                    }
+                }
+                int mval = FULL_NEG, mm = 0, mc = 0;                      // diagonal: (i-1, j-1) on k-2
+                if (i >= 1 && j >= 1 && i - 1 >= lo2 && i - 1 <= hi2) {
+                    const FullCell g = p2[i - 1 - b2];
+                    if (g.h > FULL_NEG) {
+                        const uint32_t a = ld8(tcodes + (dir > 0 ? ta + i - 1 : ta - i)), b = ld8(qcodes + (dir > 0 ? qa + j - 1 : qa - j));
+                        mval = g.h + full_sub(a, b); mm = g.hm + (a == b && a < CODE_N ? 1 : 0); mc = g.hc + 1;
+                    }
+                }
+                if (mval >= c.d && mval >= c.i) { c.h = mval; c.hm = mm; c.hc = mc; }
+                else if (c.d >= c.i) { c.h = c.d; c.hm = c.dm; c.hc = c.dc; }
+                else { c.h = c.i; c.hm = c.im; c.hc = c.ic; }
+                if (c.h <= FULL_NEG || c.h < thr) { c.h = c.d = c.i = FULL_NEG; }
+                else {
+                    if (i < nlo) nlo = i;
+                    nhi = i;
+                    if (c.h > amax) amax = c.h;
+                }
+                cur[i - clo] = c;
+            }
+            cells += (uint64_t)(chi - clo + 1);
+        }
+        syncwarp();
+        // the first cell (smallest i) that beats the best of all earlier anti-diagonals, as the sequential scan finds it
+        const int m = redmax(amax);
+        const int lo_i = redmin(nlo == INT64_MAX ? INT32_MAX : (int)nlo), hi_i = redmax(nhi == INT64_MIN ? INT32_MIN : (int)nhi);
+        if (m > best) {
+            int first = INT32_MAX;
+            for (int64_t i = clo + lane; i <= chi; i += 32) if (cur[i - clo].h == m) { first = (int)i; break; }
+            first = redmin(first);
+            const FullCell c = cur[first - clo];
+            best = m; r_score = m; r_di = first; r_dj = (int)(k - first); r_nm = c.hm; r_nc = c.hc;
+        }
+        FullCell* t = p2; p2 = p1; b2 = b1; lo2 = lo1; hi2 = hi1; p1 = cur; cur = t;
+        b1 = clo;
+        if (hi_i >= lo_i && lo_i != INT32_MAX) { lo1 = lo_i; hi1 = hi_i; } else { lo1 = 0; hi1 = -1; }
+        syncwarp();
+    }
+    if (lane == 0) {
+        res->score = r_score; res->di = r_di; res->dj = r_dj; res->nmatch = r_nm; res->ncols = r_nc;
+        res->cells = (uint32_t)(cells > 0xffffffffull ? 0xffffffffull : cells); res->status = status;
     }
 }
 

@@ -95,3 +95,23 @@ def test_hsps(T: Genome, Q: Genome, p: _lib.AlignParams):
     finally:
         _lib.lib().mb2_free_hsps(C.byref(h))
     return out, stats
+
+
+def test_seed_scan(T: Genome, Q: Genome, p: _lib.AlignParams, init_cap: int = 0):
+    """Stage (a) only (test hook): the seed hits the first-stage x-drop could not rule out, in one scan of the whole query.
+    Returns (survivors (n,2) [target, query] padded seed starts in scan order, t_off, q_off, counters[4] = survivors,
+    seed hits, leaders, stage-1 cells). init_cap: initial survivor capacity (0 = default)."""
+    s = _lib.SeedSurvivors()
+    _lib.check(_lib.lib().mb2_test_seed_scan(T.handle, Q.handle, C.byref(p), int(init_cap), C.byref(s)))
+    try:
+        n = int(s.n)
+        surv = np.zeros((n, 2), np.int64)
+        if n:
+            surv[:, 0] = np.ctypeslib.as_array(s.t_pos, shape=(n,))
+            surv[:, 1] = np.ctypeslib.as_array(s.q_pos, shape=(n,))
+        t_off = np.ctypeslib.as_array(s.t_off, shape=(int(s.t_nscaf),)).astype(np.int64)
+        q_off = np.ctypeslib.as_array(s.q_off, shape=(int(s.q_nscaf),)).astype(np.int64)
+        counters = [int(x) for x in s.counters]
+    finally:
+        _lib.lib().mb2_free_seed_survivors(C.byref(s))
+    return surv, t_off, q_off, counters

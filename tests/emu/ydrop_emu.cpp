@@ -13,11 +13,14 @@ namespace {
 struct Job {
     const uint8_t *tc, *qc; long ta, qa; int dir; yw::Params p; yw::Pool pool; yw::ExtResult* res; int max_s; int phase; uint32_t lay_mask; uint32_t priv_used = 0;
     yw::WalkCache wc;
+    long tn = 0, qn = 0; yw::FullCell* rows = nullptr; long cap = 0;
 };
 Job* g_job;
 void lane_main() {
     Job& j = *g_job;
-    if (j.phase == 0) {
+    if (j.phase == 2) {
+        yw::ydrop_full_warp(j.tc, j.qc, j.ta, j.qa, j.dir, j.tn, j.qn, j.p, j.rows, j.cap, j.res);
+    } else if (j.phase == 0) {
         if (j.max_s >= 64) yw::ydrop_forward_warp<64>(j.tc, j.qc, j.ta, j.qa, j.dir, j.p, j.pool, 0u, 0u, j.priv_used, j.res, j.lay_mask);
         else yw::ydrop_forward_warp<32>(j.tc, j.qc, j.ta, j.qa, j.dir, j.p, j.pool, 0u, 0u, j.priv_used, j.res, j.lay_mask);
     } else {
@@ -72,6 +75,21 @@ int emu_extend(const uint8_t* tc, const uint8_t* qc, long ta, long qa, int dir, 
     for (uint32_t s = 0; s < (uint32_t)yw::NSUB; s++) used += next[s] < j.pool.per_sub ? next[s] : j.pool.per_sub;
     out[0] = res.score; out[1] = res.di; out[2] = res.dj; out[3] = res.nmatch; out[4] = res.ncols; out[5] = res.status;
     out[6] = (int)res.cells; out[7] = res.kbest; out[8] = (int)used + (int)j.pool.priv; out[9] = res.max_s; out[10] = res.nlayouts;
+    return 0;
+}
+
+// The full-row fallback (ydrop_full_warp) of one extension: tn / qn = bases available from the anchor in direction dir.
+// out: score, di, dj, nmatch, ncols, status, cells
+int emu_full(const uint8_t* tc, const uint8_t* qc, long ta, long qa, int dir, long tn, long qn, int O, int E, int Y, long cap, int* out) {
+    std::vector<yw::FullCell> rows((size_t)3 * cap);
+    yw::ExtResult res;
+    memset(&res, 0, sizeof(res));
+    Job j;
+    j.tc = tc; j.qc = qc; j.ta = ta; j.qa = qa; j.dir = dir; j.p = yw::Params{O, E, Y}; j.res = &res;
+    j.tn = tn; j.qn = qn; j.rows = rows.data(); j.cap = cap;
+    g_job = &j;
+    j.phase = 2; run_warp();
+    out[0] = res.score; out[1] = res.di; out[2] = res.dj; out[3] = res.nmatch; out[4] = res.ncols; out[5] = res.status; out[6] = (int)res.cells;
     return 0;
 }
 }
