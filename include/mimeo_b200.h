@@ -277,7 +277,7 @@ MB2_API int mb2_format_gff(const int32_t* chrom, const int32_t* start, const int
                            int nnames, const char* source, const char* label, const char* prefix, uint64_t first_id, int nthreads,
                            mb2_text* out);
 
-/* ---- tandem-repeat mask of `mimeo map --maxtandem` -------------------------------------------------- */
+/* ---- tandem-repeat mask of `mimeo map --maxtandem` and `mimeo filter` ------------------------------------ */
 /* The reference runs Tandem Repeats Finder on every A-genome hit span; this build computes its own mask (DESIGN §2,
  * T1-T4; not TRF): local self-alignment of the span within diagonals 1..maxperiod, +match / -mismatch (N never matches),
  * -delta per indel; a position is masked iff it lies between the two aligned positions of a column of some such
@@ -291,15 +291,19 @@ MB2_API void mb2_default_tandem_params(mb2_tandem_params* p);
  * minscore < 1, maxperiod outside 1..256, minscore + mismatch > 65535) or a span outside its scaffold: MB2_ERR_INVALID_ARG. */
 MB2_API int mb2_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
                             const mb2_tandem_params* p, uint64_t* masked);
-/* Test hook: mb2_tandem_mask that also returns the merged masked runs of every span (span-local, closed [start, end]):
- * run r of span k is (start[r], end[r]) for off[k] <= r < off[k+1]. store_budget = bytes of device storage per launch
- * (0 = default; small values force many launches). Arrays owned by the library; free with mb2_free_tandem_runs. */
+/* mb2_tandem_mask that also returns the merged masked runs of every span (span-local, closed [start, end]): run r of span k
+ * is (start[r], end[r]) for off[k] <= r < off[k+1], runs in increasing order. Arrays owned by the library; free with
+ * mb2_free_tandem_runs (also after an error). What `mimeo filter --writeTRF` replaces by N. */
 typedef struct mb2_tandem_runs {
     uint64_t* off;       /* n + 1 entries */
     int64_t* start;
     int64_t* end;
     uint64_t n;
 } mb2_tandem_runs;
+MB2_API int mb2_tandem_mask_runs(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                                 const mb2_tandem_params* p, uint64_t* masked, mb2_tandem_runs* runs);
+/* Test hook: mb2_tandem_mask_runs with store_budget = bytes of device storage per launch (0 = default; small values force
+ * many launches). */
 MB2_API int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
                                  const mb2_tandem_params* p, uint64_t store_budget, uint64_t* masked, mb2_tandem_runs* runs);
 MB2_API void mb2_free_tandem_runs(mb2_tandem_runs* r);

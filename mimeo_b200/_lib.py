@@ -120,6 +120,8 @@ SIGNATURES = {
     'mb2_free_text': (None, [C.POINTER(Text)]),
     'mb2_default_tandem_params': (None, [C.POINTER(TandemParams)]),
     'mb2_tandem_mask': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(TandemParams), C.c_void_p]),
+    'mb2_tandem_mask_runs': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(TandemParams), C.c_void_p,
+                                       C.POINTER(TandemRuns)]),
     'mb2_test_tandem_mask': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(TandemParams), C.c_uint64,
                                        C.c_void_p, C.POINTER(TandemRuns)]),
     'mb2_free_tandem_runs': (None, [C.POINTER(TandemRuns)]),

@@ -1,14 +1,16 @@
-"""`mimeo <x|self|map>` dispatcher (host mirror of src/mimeo/app.py:21-63). The tandem-repeat filter runs inside
-`mimeo map --maxtandem` (GPU mask, DESIGN §2 T1-T4); the separate `filter` subcommand is not provided."""
+"""`mimeo <x|self|map|filter>` dispatcher (host mirror of src/mimeo/app.py:21-63). The tandem-repeat mask (GPU, DESIGN §2
+T1-T4) filters alignments in `mimeo map --maxtandem` and whole FASTA records in `mimeo filter`."""
 import sys
 from importlib import import_module
 
-COMMANDS = {'x': 'mimeo_b200.run_interspecies', 'self': 'mimeo_b200.run_self', 'map': 'mimeo_b200.run_map'}
+COMMANDS = {'x': 'mimeo_b200.run_interspecies', 'self': 'mimeo_b200.run_self', 'map': 'mimeo_b200.run_map',
+            'filter': 'mimeo_b200.run_filter'}
 
 
 def print_usage():
     print('\nUsage: mimeo <command> [options]\n\nCommands:\n  x       Run cross-species comparison\n'
-          '  self    Run self-alignment analysis\n  map     Run genomic mapping\n\nFor command-specific help:\n  mimeo <command> --help\n')
+          '  self    Run self-alignment analysis\n  map     Run genomic mapping\n'
+          '  filter  Remove tandem-repeat-rich sequences from a FASTA library\n\nFor command-specific help:\n  mimeo <command> --help\n')
 
 
 def main():

@@ -582,10 +582,10 @@ int mb2_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* sta
         tandem_mask(*g->g, scaf, start, len, n, to_tandem(p), 0, masked, nullptr);
     });
 }
-int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
-                         const mb2_tandem_params* p, uint64_t store_budget, uint64_t* masked, mb2_tandem_runs* runs) {
+static int tandem_mask_runs(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                            const mb2_tandem_params* p, uint64_t store_budget, uint64_t* masked, mb2_tandem_runs* runs) {
     return guarded([&] {
-        MB2_REQUIRE(g && g->g && runs, MB2_ERR_INVALID_ARG, "test_tandem_mask: null argument");
+        MB2_REQUIRE(g && g->g && runs, MB2_ERR_INVALID_ARG, "tandem_mask_runs: null argument");
         std::memset(runs, 0, sizeof(*runs));
         std::vector<std::vector<std::pair<int64_t, int64_t>>> iv;
         tandem_mask(*g->g, scaf, start, len, n, to_tandem(p), (size_t)store_budget, masked, &iv);
@@ -594,7 +594,7 @@ int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t
         runs->off = (uint64_t*)malloc((n + 1) * sizeof(uint64_t));
         runs->start = (int64_t*)malloc((total ? total : 1) * sizeof(int64_t));
         runs->end = (int64_t*)malloc((total ? total : 1) * sizeof(int64_t));
-        MB2_REQUIRE(runs->off && runs->start && runs->end, MB2_ERR_INTERNAL, "test_tandem_mask: host allocation failed");
+        MB2_REQUIRE(runs->off && runs->start && runs->end, MB2_ERR_INTERNAL, "tandem_mask_runs: host allocation failed");
         runs->n = n;
         runs->off[0] = 0;
         for (uint64_t k = 0; k < n; k++) {
@@ -605,6 +605,14 @@ int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t
             runs->off[k + 1] = runs->off[k] + iv[k].size();
         }
     });
+}
+int mb2_tandem_mask_runs(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                         const mb2_tandem_params* p, uint64_t* masked, mb2_tandem_runs* runs) {
+    return tandem_mask_runs(g, scaf, start, len, n, p, 0, masked, runs);
+}
+int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                         const mb2_tandem_params* p, uint64_t store_budget, uint64_t* masked, mb2_tandem_runs* runs) {
+    return tandem_mask_runs(g, scaf, start, len, n, p, store_budget, masked, runs);
 }
 void mb2_free_tandem_runs(mb2_tandem_runs* r) {
     if (!r) return;

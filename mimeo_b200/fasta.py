@@ -46,20 +46,25 @@ def read_fasta(path: str, nthreads: int = 0) -> List[Tuple[str, str, np.ndarray]
     return out
 
 
-def write_fasta_record(path: str, header: str, seq: np.ndarray, width: int = 60) -> None:
-    """One record, sequence wrapped at `width` columns (SeqIO.write's layout)."""
+def write_fasta_record(path, header: str, seq: np.ndarray, width: int = 60) -> None:
+    """One record, sequence wrapped at `width` columns (SeqIO.write's layout). `path` is a file name, which then holds
+    this record alone, or a binary file open for writing, to which the record is appended (many records, one file)."""
+    if not hasattr(path, 'write'):
+        with open(path, 'wb') as f:
+            write_fasta_record(f, header, seq, width)
+        return
+    f = path
     n = len(seq)
-    with open(path, 'wb') as f:
-        f.write(b'>' + header.encode() + b'\n')
-        if n:
-            full = n // width
-            if full:
-                block = np.empty((full, width + 1), dtype=np.uint8)
-                block[:, :width] = seq[:full * width].reshape(full, width)
-                block[:, width] = 10
-                f.write(block.tobytes())
-            if n % width:
-                f.write(seq[full * width:].tobytes() + b'\n')
+    f.write(b'>' + header.encode() + b'\n')
+    if n:
+        full = n // width
+        if full:
+            block = np.empty((full, width + 1), dtype=np.uint8)
+            block[:, :width] = seq[:full * width].reshape(full, width)
+            block[:, width] = 10
+            f.write(block.tobytes())
+        if n % width:
+            f.write(seq[full * width:].tobytes() + b'\n')
 
 
 def dir_records(seqdir: str) -> Iterator[Tuple[str, str, np.ndarray, str]]:

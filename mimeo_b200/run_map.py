@@ -2,7 +2,7 @@
 that percentage are dropped after numbering (import_Align -> tandem filter -> GFF3, SURVEY 3.3), so the surviving rows
 keep their IDs. The mask is this project's own GPU statement (DESIGN §2, T1-T4), not Tandem Repeats Finder: --TRFpath,
 --tPM and --tPI are accepted and have no effect. --writeTRF (with --maxtandem) also writes the .tab lines of the surviving
-hits to `<outfile without .tab>_TRFfiltered.tab`."""
+hits to `<outfile without .tab>_TRFfiltered.tab`. The same mask filters whole FASTA records in `mimeo filter` (run_filter.py)."""
 import argparse
 import logging
 import os

@@ -1,10 +1,11 @@
-"""The tandem-repeat filter of `mimeo map --maxtandem` (the reference's trfFilter step, SURVEY 3.3). The mask is this
-project's own statement computed on the GPU (DESIGN §2, T1-T4; `mb2_tandem_mask`), not Tandem Repeats Finder."""
+"""The tandem-repeat filters: `mimeo map --maxtandem` (the reference's trfFilter step, SURVEY 3.3) and `mimeo filter` (its
+trfFasta step, SURVEY 3.5). The mask is this project's own statement computed on the GPU (DESIGN §2, T1-T4;
+`mb2_tandem_mask`), not Tandem Repeats Finder."""
 from __future__ import annotations
 
 import ctypes as C
 import logging
-from typing import Dict, List, Sequence, Tuple
+from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -59,21 +60,54 @@ def masked_counts(genome, scaf, start0, length, p: Dict[str, int]) -> np.ndarray
             g.close()
 
 
-def masked_runs(genome, scaf, start0, length, p: Dict[str, int], store_budget: int = 0) -> Tuple[np.ndarray, List[List[Tuple[int, int]]]]:
-    """Test hook: (masked counts, merged masked runs of every span as span-local closed (start, end) pairs)."""
-    s, b, n = _spans(scaf, start0, length)
-    out = np.zeros(len(s), dtype=np.uint64)
+def _with_runs(nspans: int, call) -> Tuple[np.ndarray, List[List[Tuple[int, int]]]]:
+    """Runs call(masked, runs) on an mb2_tandem_runs result and returns (masked counts, runs of every span as lists of
+    span-local closed (start, end) pairs); the library's arrays are freed whatever happens."""
+    out = np.zeros(nspans, dtype=np.uint64)
     r = _lib.TandemRuns()
-    _lib.check(_lib.lib().mb2_test_tandem_mask(genome.handle, s.ctypes.data, b.ctypes.data, n.ctypes.data, len(s), C.byref(_cparams(p)),
-                                               int(store_budget), out.ctypes.data, C.byref(r)))
     try:
-        off = np.ctypeslib.as_array(r.off, shape=(len(s) + 1,)).copy()
+        _lib.check(call(out.ctypes.data, C.byref(r)))
+        off = np.ctypeslib.as_array(r.off, shape=(nspans + 1,)).copy()
         tot = int(off[-1])
         st = np.ctypeslib.as_array(r.start, shape=(max(tot, 1),))[:tot].tolist()
         en = np.ctypeslib.as_array(r.end, shape=(max(tot, 1),))[:tot].tolist()
     finally:
         _lib.lib().mb2_free_tandem_runs(C.byref(r))
-    return out, [list(zip(st[off[k]:off[k + 1]], en[off[k]:off[k + 1]])) for k in range(len(s))]
+    return out, [list(zip(st[off[k]:off[k + 1]], en[off[k]:off[k + 1]])) for k in range(nspans)]
+
+
+def masked_runs(genome, scaf, start0, length, p: Dict[str, int], store_budget: int = 0) -> Tuple[np.ndarray, List[List[Tuple[int, int]]]]:
+    """Test hook: (masked counts, merged masked runs of every span as span-local closed (start, end) pairs)."""
+    s, b, n = _spans(scaf, start0, length)
+    return _with_runs(len(s), lambda m, r: _lib.lib().mb2_test_tandem_mask(genome.handle, s.ctypes.data, b.ctypes.data, n.ctypes.data,
+                                                                            len(s), C.byref(_cparams(p)), int(store_budget), m, r))
+
+
+def record_masks(seqs: Sequence[np.ndarray], p: Dict[str, int], runs: bool = False) -> Tuple[np.ndarray, Optional[List[List[Tuple[int, int]]]]]:
+    """`mimeo filter`: the masked positions of every record, each masked as one span [0, L), and with runs=True also its
+    merged masked runs (closed (start, end) pairs; None otherwise). The records with L >= 1 go to the device as one Genome;
+    a record with L = 0 never does (m = 0, no runs)."""
+    from .genome import Genome
+    lens = np.array([len(s) for s in seqs], dtype=np.int64)
+    idx = np.flatnonzero(lens > 0)
+    m = np.zeros(len(seqs), dtype=np.uint64)
+    iv: Optional[List[List[Tuple[int, int]]]] = [[] for _ in seqs] if runs else None
+    if not len(idx):
+        return m, iv
+    g = Genome([str(k) for k in idx.tolist()], [seqs[k] for k in idx.tolist()])
+    try:
+        s, b, n = _spans(np.arange(len(idx)), np.zeros(len(idx)), lens[idx])
+        if runs:
+            got, got_iv = _with_runs(len(s), lambda mm, r: _lib.lib().mb2_tandem_mask_runs(g.handle, s.ctypes.data, b.ctypes.data, n.ctypes.data,
+                                                                                          len(s), C.byref(_cparams(p)), mm, r))
+            for k, v in zip(idx.tolist(), got_iv):
+                iv[k] = v
+        else:
+            got = masked_counts(g, s, b, n, p)
+    finally:
+        g.close()
+    m[idx] = got
+    return m, iv
 
 
 def _tab_key(fields: Sequence[str]) -> Tuple[str, ...]:
@@ -149,3 +183,39 @@ def trf_path(outtab: str) -> str:
     """`<outfile without .tab>_TRFfiltered.tab`."""
     stem = outtab[:-4] if outtab.endswith('.tab') else outtab
     return stem + '_TRFfiltered.tab'
+
+
+def write_filtered_fasta(records: Sequence[Tuple[str, str, np.ndarray]], outfile: str, maxtandem: float, p: Dict[str, int],
+                         masked_out: str = None) -> int:
+    """`mimeo filter`: of the (id, header, seq) records, write to outfile, in input order, every record unless more than
+    maxtandem percent of it is masked (a record with L = 0 is kept); with masked_out also write every record there with its
+    masked positions replaced by N. Both files in SeqIO.write's layout. Returns the number of records kept."""
+    from .fasta import write_fasta_record
+    seqs = [r[2] for r in records]
+    m, runs = record_masks(seqs, p, runs=masked_out is not None)
+    keep = [len(s) == 0 or not (100.0 * float(mm) / len(s) > maxtandem) for s, mm in zip(seqs, m.tolist())]
+    with open(outfile, 'wb') as f:
+        for (_rid, header, seq), k in zip(records, keep):
+            if k:
+                write_fasta_record(f, header, seq)
+    if masked_out is not None:
+        with open(masked_out, 'wb') as f:
+            for (_rid, header, seq), iv in zip(records, runs):
+                if iv:
+                    seq = seq.copy()
+                    for a, e in iv:
+                        seq[a:e + 1] = ord('N')
+                write_fasta_record(f, header, seq)
+    kept = sum(keep)
+    logging.info('Tandem repeat filter: %d of %d records kept (maxtandem %s%%)', kept, len(records), maxtandem)
+    if not kept:
+        logging.warning('Every record was removed by the tandem repeat filter; %s is empty.', outfile)
+    return kept
+
+
+def masked_fasta_path(outfile: str) -> str:
+    """`<outfile without .fa/.fasta/.fna>_TRFmasked.fa`."""
+    for ext in ('.fa', '.fasta', '.fna'):
+        if outfile.endswith(ext):
+            return outfile[:-len(ext)] + '_TRFmasked.fa'
+    return outfile + '_TRFmasked.fa'
