@@ -113,6 +113,9 @@ MB2_API int mb2_genome_both_strands(const mb2_genome* g, mb2_genome** out);
 MB2_API void mb2_genome_free(mb2_genome* g);
 /* Test hook: scaffold `scaf` decoded back to codes 0..3 = ACGT, 4 = other (HOST buffer of its length). */
 MB2_API int mb2_genome_decode(const mb2_genome* g, int scaf, uint8_t* out);
+/* Test hook: the 4-bit code plane of the whole padded coordinate space (8 codes per word). Sets *nwords to its length in
+ * words and copies min(cap, *nwords) words to the HOST buffer out (out may be null when cap is 0). */
+MB2_API int mb2_test_genome_nibbles(const mb2_genome* g, uint32_t* out, uint64_t cap, uint64_t* nwords);
 
 /* ---- alignment parameters --------------------------------------------------------------- */
 /* The knobs of the one LASTZ command line mimeo issues (wrappers.py:1031): --hspthresh is the only

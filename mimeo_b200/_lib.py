@@ -92,6 +92,7 @@ SIGNATURES = {
     'mb2_genome_both_strands': (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
     'mb2_genome_free': (None, [C.c_void_p]),
     'mb2_genome_decode': (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    'mb2_test_genome_nibbles': (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
     'mb2_default_align_params': (None, [C.POINTER(AlignParams)]),
     'mb2_free_hsps': (None, [C.POINTER(Hsps)]),
     'mb2_test_hsps': (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(AlignParams), C.POINTER(Hsps), C.c_void_p]),

@@ -329,6 +329,17 @@ int mb2_genome_decode(const mb2_genome* g, int scaf, uint8_t* out) {
         genome_decode(*g->g, scaf, out);
     });
 }
+int mb2_test_genome_nibbles(const mb2_genome* g, uint32_t* out, uint64_t cap, uint64_t* nwords) {
+    return guarded([&] {
+        ensure_init();
+        MB2_REQUIRE(g && g->g && nwords && (out || cap == 0), MB2_ERR_INVALID_ARG, "test_genome_nibbles: null argument");
+        const uint64_t n = g->g->G / 8 + 8;
+        *nwords = n;
+        const uint64_t k = cap < n ? cap : n;
+        if (k) MB2_CUDA(cudaMemcpyAsync(out, g->g->nb.get(), k * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx().stream));
+        MB2_CUDA(cudaStreamSynchronize(ctx().stream));
+    });
+}
 
 void mb2_default_align_params(mb2_align_params* p) {
     if (!p) return;

@@ -1,4 +1,4 @@
-// genome.cu -- build the device genome (2-bit pack + N mask) from ASCII, and its reverse complement.
+// genome.cu -- build the device genome (2-bit pack, N mask, 4-bit codes) from ASCII, and its reverse complement.
 // Replaces the FASTA -> per-scaffold files -> LASTZ sequence loading of the reference
 // (utils.py:274-309 splitFasta, LASTZ's own reader) for the hot path.
 #include "seq.cuh"
@@ -12,10 +12,18 @@ __device__ __forceinline__ uint32_t code_byte(uint32_t base, uint32_t bad, uint3
     return pad ? 12u : (bad ? 8u : (base | (((base ^ (base >> 1)) & 1u) << 2)));
 }
 
-// one thread packs 32 bases -> one uint64 of 2-bit codes + one uint32 of N flags
+// the four nb words of 32 bases (2-bit codes `bits`, non-ACGT flags `nflag`)
+__device__ __forceinline__ void store_nibbles(uint32_t* __restrict__ nb, uint32_t w, uint64_t bits, uint32_t nflag) {
+    uint32_t v[4] = {0, 0, 0, 0};
+#pragma unroll
+    for (int c = 0; c < 32; c++) v[c >> 3] |= nib_code((uint32_t)(bits >> (2 * c)) & 3u, (nflag >> c) & 1u) << (4 * (c & 7));
+    reinterpret_cast<uint4*>(nb)[w] = make_uint4(v[0], v[1], v[2], v[3]);
+}
+
+// one thread packs 32 bases -> one uint64 of 2-bit codes + one uint32 of N flags (+ soft-mask flags, 4-bit codes, code bytes)
 __global__ void __launch_bounds__(256)
 pack_kernel(const uint8_t* __restrict__ ascii, uint32_t nwords, uint64_t* __restrict__ pk, uint32_t* __restrict__ nm,
-            uint32_t* __restrict__ sm, uint8_t* __restrict__ codes, int* __restrict__ any_soft) {
+            uint32_t* __restrict__ sm, uint32_t* __restrict__ nb, uint8_t* __restrict__ codes, int* __restrict__ any_soft) {
     const uint32_t w = blockIdx.x * blockDim.x + threadIdx.x;
     if (w >= nwords) return;
     const uint4* src = reinterpret_cast<const uint4*>(ascii + (size_t)w * 32);
@@ -44,6 +52,7 @@ pack_kernel(const uint8_t* __restrict__ ascii, uint32_t nwords, uint64_t* __rest
     pk[w] = bits;
     nm[w] = nflag;
     sm[w] = nflag | lowflag;
+    store_nibbles(nb, w, bits, nflag);
     if (lowflag & ~nflag) atomicOr(any_soft, 1);      // rare: only soft-masked assemblies take this
     uint32_t out[8];
 #pragma unroll
@@ -63,7 +72,8 @@ pack_kernel(const uint8_t* __restrict__ ascii, uint32_t nwords, uint64_t* __rest
 
 // reverse complement every scaffold in place of its own slot (same offsets, same lengths)
 __global__ void __launch_bounds__(256)
-revcomp_kernel(GenomeView src, uint64_t* __restrict__ pk, uint32_t* __restrict__ nm, uint32_t* __restrict__ sm, uint8_t* __restrict__ codes, uint32_t nwords) {
+revcomp_kernel(GenomeView src, uint64_t* __restrict__ pk, uint32_t* __restrict__ nm, uint32_t* __restrict__ sm, uint32_t* __restrict__ nb,
+               uint8_t* __restrict__ codes, uint32_t nwords) {
     const uint32_t w = blockIdx.x * blockDim.x + threadIdx.x;
     if (w >= nwords) return;
     const uint32_t p0 = w * 32;
@@ -90,6 +100,7 @@ revcomp_kernel(GenomeView src, uint64_t* __restrict__ pk, uint32_t* __restrict__
     pk[w] = bits;
     nm[w] = nflag;
     sm[w] = sflag;
+    store_nibbles(nb, w, bits, nflag);
 }
 
 // nfree[s] = 1 iff scaffold s has no non-ACGT base (one CTA per scaffold scans its mask words)
@@ -140,13 +151,13 @@ Genome* genome_from_ascii(const uint8_t* const* seqs, const uint64_t* lens, int 
         for (int s = 0; s < n; s++)
             if (lens[s]) MB2_CUDA(cudaMemcpyAsync(d_ascii.get() + g->off[s], seqs[s], lens[s], cudaMemcpyHostToDevice, cx.stream));
         const uint32_t nwords = (uint32_t)(g->G / 32) + 2;
-        g->pk.alloc(nwords); g->nm.alloc(nwords); g->sm.alloc(nwords); g->codes.alloc((size_t)nwords * 32);
+        g->pk.alloc(nwords); g->nm.alloc(nwords); g->sm.alloc(nwords); g->nb.alloc((size_t)nwords * 4); g->codes.alloc((size_t)nwords * 32);
         g->d_off.alloc(n); g->d_len.alloc(n);
         MB2_CUDA(cudaMemcpyAsync(g->d_off.get(), g->off.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, cx.stream));
         MB2_CUDA(cudaMemcpyAsync(g->d_len.get(), g->len.data(), n * sizeof(uint32_t), cudaMemcpyHostToDevice, cx.stream));
         DevBuf<int> d_soft(1);
         MB2_CUDA(cudaMemsetAsync(d_soft.get(), 0, sizeof(int), cx.stream));
-        launch(pack_kernel, cdiv(nwords, 256), 256, 0, d_ascii.get(), nwords, g->pk.get(), g->nm.get(), g->sm.get(), g->codes.get(), d_soft.get());
+        launch(pack_kernel, cdiv(nwords, 256), 256, 0, d_ascii.get(), nwords, g->pk.get(), g->nm.get(), g->sm.get(), g->nb.get(), g->codes.get(), d_soft.get());
         int h_soft = 0;
         MB2_CUDA(cudaMemcpyAsync(&h_soft, d_soft.get(), sizeof(int), cudaMemcpyDeviceToHost, cx.stream));
         g->d_nfree.alloc(n);
@@ -165,14 +176,14 @@ Genome* genome_revcomp(const Genome& src) {
         g->nscaf = src.nscaf; g->off = src.off; g->len = src.len; g->G = src.G; g->nbases = src.nbases; g->is_rc = !src.is_rc;
         g->has_soft = src.has_soft;
         const uint32_t nwords = (uint32_t)(g->G / 32) + 2;
-        g->pk.alloc(nwords); g->nm.alloc(nwords); g->sm.alloc(nwords); g->codes.alloc((size_t)nwords * 32);
+        g->pk.alloc(nwords); g->nm.alloc(nwords); g->sm.alloc(nwords); g->nb.alloc((size_t)nwords * 4); g->codes.alloc((size_t)nwords * 32);
         g->d_off.alloc(src.nscaf); g->d_len.alloc(src.nscaf);
         Ctx& cx = ctx();
         MB2_CUDA(cudaMemcpyAsync(g->d_off.get(), src.d_off.get(), src.nscaf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, cx.stream));
         MB2_CUDA(cudaMemcpyAsync(g->d_len.get(), src.d_len.get(), src.nscaf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, cx.stream));
         g->d_nfree.alloc(src.nscaf);
         MB2_CUDA(cudaMemcpyAsync(g->d_nfree.get(), src.d_nfree.get(), src.nscaf * sizeof(uint32_t), cudaMemcpyDeviceToDevice, cx.stream));
-        launch(revcomp_kernel, cdiv(nwords, 256), 256, 0, view(src), g->pk.get(), g->nm.get(), g->sm.get(), g->codes.get(), nwords);
+        launch(revcomp_kernel, cdiv(nwords, 256), 256, 0, view(src), g->pk.get(), g->nm.get(), g->sm.get(), g->nb.get(), g->codes.get(), nwords);
         g->id = next_genome_id(); g->fwd_src_id = 0; g->nfwd = 0;
     } catch (...) { delete g; throw; }
     return g;
@@ -182,7 +193,8 @@ Genome* genome_revcomp(const Genome& src) {
 // alignment pipeline cover --strand=both (tile = target x (scaffold, strand)), so the two strands share every launch.
 __global__ void __launch_bounds__(256)
 both_strands_kernel(GenomeView src, const uint32_t* __restrict__ noff, const uint32_t* __restrict__ nlen, int n2,
-                    uint64_t* __restrict__ pk, uint32_t* __restrict__ nm, uint32_t* __restrict__ sm, uint8_t* __restrict__ codes, uint32_t nwords) {
+                    uint64_t* __restrict__ pk, uint32_t* __restrict__ nm, uint32_t* __restrict__ sm, uint32_t* __restrict__ nb,
+                    uint8_t* __restrict__ codes, uint32_t nwords) {
     const uint32_t w = blockIdx.x * blockDim.x + threadIdx.x;
     if (w >= nwords) return;
     const uint32_t p0 = w * 32;
@@ -210,6 +222,7 @@ both_strands_kernel(GenomeView src, const uint32_t* __restrict__ noff, const uin
         cw[c >> 2] |= code_byte(code, bad, (p >= so && p < so + sl) ? 0u : 1u) << (8 * (c & 3));
     }
     pk[w] = bits; nm[w] = nflag; sm[w] = sflag;
+    store_nibbles(nb, w, bits, nflag);
     uint4* dst = reinterpret_cast<uint4*>(codes + (size_t)w * 32);
     dst[0] = make_uint4(cw[0], cw[1], cw[2], cw[3]);
     dst[1] = make_uint4(cw[4], cw[5], cw[6], cw[7]);
@@ -224,7 +237,7 @@ Genome* genome_both_strands(const Genome& src) {
         layout(*g, lens.data(), 2 * n);
         g->has_soft = src.has_soft;
         const uint32_t nwords = (uint32_t)(g->G / 32) + 2;
-        g->pk.alloc(nwords); g->nm.alloc(nwords); g->sm.alloc(nwords); g->codes.alloc((size_t)nwords * 32);
+        g->pk.alloc(nwords); g->nm.alloc(nwords); g->sm.alloc(nwords); g->nb.alloc((size_t)nwords * 4); g->codes.alloc((size_t)nwords * 32);
         g->d_off.alloc(2 * n); g->d_len.alloc(2 * n); g->d_nfree.alloc(2 * n);
         Ctx& cx = ctx();
         MB2_CUDA(cudaMemcpyAsync(g->d_off.get(), g->off.data(), 2 * n * sizeof(uint32_t), cudaMemcpyHostToDevice, cx.stream));
@@ -232,7 +245,7 @@ Genome* genome_both_strands(const Genome& src) {
         MB2_CUDA(cudaMemcpyAsync(g->d_nfree.get(), src.d_nfree.get(), n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, cx.stream));
         MB2_CUDA(cudaMemcpyAsync(g->d_nfree.get() + n, src.d_nfree.get(), n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, cx.stream));
         launch(both_strands_kernel, cdiv(nwords, 256), 256, 0, view(src), g->d_off.get(), g->d_len.get(), 2 * n, g->pk.get(), g->nm.get(),
-               g->sm.get(), g->codes.get(), nwords);
+               g->sm.get(), g->nb.get(), g->codes.get(), nwords);
         MB2_CUDA(cudaStreamSynchronize(cx.stream));   // g->off/len host vectors were copy sources
         g->id = next_genome_id(); g->fwd_src_id = src.fwd_src_id == src.id ? src.id : 0; g->nfwd = src.fwd_src_id == src.id ? n : 0;
     } catch (...) { delete g; throw; }

@@ -23,10 +23,9 @@ namespace mb2 {
 
 constexpr uint32_t KEY_INVALID = 1u << 24;
 constexpr int S1_WINDOW = 30;        // columns per first-stage window = 10 table chunks of 3 columns
-constexpr uint32_t S1_WINDOW_MASK = (1u << S1_WINDOW) - 1u;
 constexpr int S1_RIGHT_WINDOWS = 2;  // 60 columns
 constexpr int S1_LEFT_WINDOWS = 3;   // 90 columns (19 of them are the seed itself)
-constexpr int S1_TAB = XT_SIZE;      // (3 target bases, 3 query bases) -> packed {sum, first argmax, max prefix, min prefix}
+constexpr int S1_TAB = XT_SIZE;      // 3 columns of merged 4-bit codes -> packed {sum, max prefix, min prefix}
 
 __global__ void __launch_bounds__(256)
 seed_keys_kernel(GenomeView T, uint32_t p_lo, uint32_t n, uint32_t* __restrict__ keys, uint32_t* __restrict__ pos) {
@@ -60,57 +59,63 @@ void build_seed_table(const Genome& T, uint32_t p_lo, uint32_t p_hi, SeedTable& 
     tab.p_lo = p_lo; tab.p_hi = p_hi;
 }
 
-// First-stage table: the three-column entry of xdrop_table.cuh with the x-drop baked in and no argmax field, so that a chunk
-// costs no constant arithmetic:  bits 22..31 = s0+s1+s2 (signed), bits 13..21 = 125 + max prefix sum,
-// bits 0..12 = 125 + X + min prefix sum.  State of a lane: (best, D) with D = (best - run) + 125 >= 125; a chunk is
+// First-stage table over merged codes: three columns of 4 bits, m = t ^ q on the base bits and t | q on the parity and
+// non-ACGT bits (nib_merge). That is enough to score a column: a set bit 3 scores SCORE_N; otherwise x = t ^ q decides HOXD70
+// except for x = 0 (A/A 91, C/C 100) and x = 3 (A/T -123, C/G -125), whose two bases have equal parity, so the OR is the target's.
+// N columns inside the table keep the chunk rule exact (-100 lies within HOXD70's range: prefix sums inside a chunk still differ
+// by at most 250 < X). Entry: bits 22..31 = s0+s1+s2 (signed), bits 13..21 = 125 + max prefix sum, bits 0..12 = 125 + X + min
+// prefix sum. State of a lane: (best, D) with D = (best - run) + 125 >= 125; a chunk is
 //   terminate iff min_field < D;   DM = max(D, max_field);   best += DM - D;   D = DM - sum
 // (the rule of xdrop_table.cuh with D shifted by X - 250). A finished lane parks at D = S1_DONE, where every later chunk is
 // a no-op on best.
+// The index of a chunk is its 12 bits of merged code with bits 2..3 (parity and N of the first column) xor bits 8..9 (x of the
+// third column; s1_prepare). The bank of a lookup is index bits 0..4, and the 32 hits of a batch mostly share one query
+// window: of the plain code only x of the first column and one bit of x of the second vary with the target there (8 banks,
+// about 5.2 wavefronts per lookup for random bases against 2.0 for 32 banks); with the xor all five bits do.
 constexpr int S1_DONE = 1 << 24;
 constexpr int S1_D0 = 125;                     // run = best = 0
 constexpr int S1_MAX_XDROP = 8191 - 125 - 300; // min field fits 13 bits
 __device__ __forceinline__ uint32_t s1_entry(uint32_t idx, int X) {
-    const uint32_t q6 = idx >> 6, t6 = idx & 63;
+    const uint32_t code = idx ^ (((idx >> 8) & 3u) << 2);
     int sum = 0, mx = INT_MIN, mn = INT_MAX;
     for (int c = 0; c < 3; c++) {
-        sum += sub_lut((((t6 >> (2 * c)) & 3u) << 2) | ((q6 >> (2 * c)) & 3u));
+        const uint32_t nib = (code >> (4 * c)) & 15u, t = (nib >> 2) & 1u;   // t: A or C, with the column's parity
+        sum += (nib & 8u) ? SCORE_N : sub_lut((t << 2) | (t ^ (nib & 3u)));
         mx = max(mx, sum); mn = min(mn, sum);
     }
     return ((uint32_t)sum << 22) | ((uint32_t)(mx + 125) << 13) | (uint32_t)(mn + X + 125);
 }
-// bits [s, s + 32) of the 64-bit word (hi:lo) for a compile-time s in (-32, 64); negative s shifts left
-__device__ __forceinline__ uint32_t s1_bits(uint32_t lo, uint32_t hi, int s) {
-    return s <= 0 ? lo << (-s) : (s < 32 ? __funnelshift_r(lo, hi, s) : hi >> (s - 32));
+// bits [s, s + 32) of the 128-bit window w for a compile-time s in (-32, 128); negative s shifts left
+__device__ __forceinline__ uint32_t s1_bits(const uint32_t (&w)[4], int s) {
+    if (s < 0) return w[0] << (-s);
+    const int j = s >> 5, r = s & 31;
+    return r == 0 ? w[j] : (j < 3 ? __funnelshift_r(w[j], w[j + 1], r) : w[3] >> r);
 }
-// 30 columns (first column in the low bits of wt / wq / an); updates (best, D) of the lane exactly as the
-// column-by-column rule would. Lanes whose window holds a non-ACGT column take the per-column path.
-// tab_sa = shared-space address of the table. nchunks counts the chunks a lane entered while still open.
+// A window of merged codes (first column in the low bits of w[0]) made ready for xdrop_window30: returns whether one of its
+// 30 columns is non-ACGT, then applies the index xor of every chunk.
+__device__ __forceinline__ bool s1_prepare(uint32_t (&w)[4]) {
+    const bool an = (((w[0] | w[1] | w[2]) & 0x88888888u) | (w[3] & 0x00888888u)) != 0;
+    constexpr uint32_t SW0 = 0x0C00C00Cu, SW1 = 0xC00C00C0u, SW2 = 0x00C00C00u, SW3 = 0x0000C00Cu;   // bits 12k + 2, 12k + 3
+    w[0] ^= __funnelshift_r(w[0], w[1], 6) & SW0;
+    w[1] ^= __funnelshift_r(w[1], w[2], 6) & SW1;
+    w[2] ^= __funnelshift_r(w[2], w[3], 6) & SW2;
+    w[3] ^= (w[3] >> 6) & SW3;
+    return an;
+}
+// 30 columns of a prepared window; updates (best, D) of the lane exactly as the column-by-column rule would.
+// tab_sa = shared-space address of the table. nchunks counts the chunks a lane entered while still open, except that a window
+// with a non-ACGT column (an) that is entered while open counts all 10 (the count the scan has always reported).
 template <uint32_t VOTES>
-__device__ __forceinline__ void xdrop_window30(uint32_t tab_sa, uint32_t m10, uint32_t m9, uint64_t wt, uint64_t wq, uint32_t an, int X,
+__device__ __forceinline__ void xdrop_window30(uint32_t tab_sa, uint32_t m10, uint32_t m9, const uint32_t (&w)[4], bool an,
                                                int& best, int& D, uint32_t& nchunks) {
-    int d_keep = 0;
-    bool slow = false;
-    if (D < S1_DONE / 2 && an) {
-        int run = best - (D - 125);
-        bool term = false;
-        for (int c = 0; c < S1_WINDOW && !term; c++) {
-            const int sc = (an & 1u) ? SCORE_N : sub_lut((uint32_t)((wt & 3) << 2 | (wq & 3)));
-            wt >>= 2; wq >>= 2; an >>= 1;
-            run += sc;
-            if (run > best) best = run; else if (run < best - X) term = true;
-        }
-        nchunks += S1_WINDOW / 3;
-        d_keep = term ? S1_DONE : (best - run) + 125;
-        slow = true; D = S1_DONE;              // the window is consumed: the table loop below is a no-op for this lane
-    }
-    const uint32_t tl = (uint32_t)wt, th = (uint32_t)(wt >> 32), ql = (uint32_t)wq, qh = (uint32_t)(wq >> 32);
+    const bool all10 = an && D < S1_DONE / 2;
     uint32_t parked = 0;                       // sum of D at chunk entry: S1_DONE per parked chunk + (< 2^24 in total) for the open ones
     int entered = S1_WINDOW / 3;
 #pragma unroll
     for (int k = 0; k < S1_WINDOW / 3; k++) {
         if ((VOTES >> k) & 1u) { if (__all_sync(0xffffffffu, D >= S1_DONE / 2)) { entered = k; break; } }
-        // byte address = table + (q6 << 8 | t6 << 2)
-        const uint32_t addr = ((s1_bits(tl, th, 6 * k - 2) & 0xFCu) | (s1_bits(ql, qh, 6 * k - 8) & 0x3F00u)) + tab_sa;
+        // byte address = table + 4 * (12 bits of chunk k)
+        const uint32_t addr = (s1_bits(w, 12 * k - 2) & 0x3FFCu) + tab_sa;
         uint32_t e;
         asm("ld.shared.u32 %0, [%1];" : "=r"(e) : "r"(addr));
         parked += (uint32_t)D;
@@ -122,8 +127,7 @@ __device__ __forceinline__ void xdrop_window30(uint32_t tab_sa, uint32_t m10, ui
         best += dm - D;
         D = term ? S1_DONE : dm - __mulhi((int)e, (int)m10);
     }
-    nchunks += (uint32_t)entered - (parked >> 24);
-    if (slow) D = d_keep;
+    nchunks += all10 ? (uint32_t)(S1_WINDOW / 3) : (uint32_t)entered - (parked >> 24);
 }
 // (best, D) of one side in a deferred record: best < 2^16 (at most 90 columns of at most +100), an open D < 2^13 (the min
 // field); a terminated side stores 0xFFFF in the D half.
@@ -135,54 +139,35 @@ __device__ __forceinline__ void s1_unpack(uint32_t w, int& best, int& D) {
     D = (w >> 16) == 0xFFFFu ? S1_DONE : (int)(w >> 16);
 }
 
-// 128 columns of one sequence in registers, starting at the 64-column boundary at or below `first`: packed bases, non-ACGT
-// flags and (when the genome is soft-masked) the not-seedable flags.
-struct SeqBlock {
-    uint64_t w[4];
-    uint32_t n[4], s[4];
-    uint32_t c0;
-    // The three windows a batch needs, cut out together: f = 32 columns from p (p = hit - 13: the first left window),
-    // l = from p + 12 (the leader window, hit - 1), r = from p + 32 (the first right window, hit + 19); non-ACGT flags of f
-    // and r, not-seedable flags of l. p lies in [c0, c0 + 64). The eight 32-bit words of the block are shifted by whole
-    // words with two levels of selects (shared between the outputs), then by bits with funnel shifts.
-    __device__ __forceinline__ void windows(uint32_t p, uint64_t& f, uint64_t& l, uint64_t& r, uint32_t& fn, uint32_t& rn, uint32_t& ls) const {
-        const uint32_t off = p - c0, sh = (off & 15u) * 2u;
-        const bool b0 = off & 16u, b1 = off & 32u;
-        uint32_t x[8], a[7], y[5];
+// Merged code of target and query nb words (see s1_entry): one LOP3
+__device__ __forceinline__ uint32_t nib_merge(uint32_t t, uint32_t q) {
+    return ((t ^ q) & 0x33333333u) | ((t | q) & 0xCCCCCCCCu);
+}
+// the eight 4-bit groups of a word in reverse order
+__device__ __forceinline__ uint32_t nib_rev(uint32_t x) {
+    x = __byte_perm(x, 0u, 0x0123u);
+    return ((x >> 4) & 0x0F0F0F0Fu) | ((x << 4) & 0xF0F0F0F0u);
+}
+// NW words of nb codes = the 8 NW columns from column p (p in the low bits of w[0]), read as NW / 2 + 1 aligned 8-byte loads
+template <int NW>
+__device__ __forceinline__ void nib_span(const uint32_t* __restrict__ nb, uint32_t p, uint32_t (&w)[NW]) {
+    const uint32_t w0 = (p >> 3) & ~1u, sh = (p & 7u) * 4u;
+    const bool odd = p & 8u;
+    uint32_t x[NW + 2];
 #pragma unroll
-        for (int m = 0; m < 4; m++) { x[2 * m] = (uint32_t)w[m]; x[2 * m + 1] = (uint32_t)(w[m] >> 32); }
-#pragma unroll
-        for (int m = 0; m < 7; m++) a[m] = b0 ? x[m + 1] : x[m];
-#pragma unroll
-        for (int m = 0; m < 5; m++) y[m] = b1 ? a[m + 2] : a[m];
-        const uint32_t f0 = __funnelshift_r(y[0], y[1], sh), f1 = __funnelshift_r(y[1], y[2], sh);
-        const uint32_t r0 = __funnelshift_r(y[2], y[3], sh), r1 = __funnelshift_r(y[3], y[4], sh);
-        f = (uint64_t)f0 | ((uint64_t)f1 << 32); r = (uint64_t)r0 | ((uint64_t)r1 << 32);
-        l = (uint64_t)__funnelshift_r(f0, f1, 24) | ((uint64_t)__funnelshift_r(f1, r0, 24) << 32);
-        const uint32_t sn = off & 31u;
-        const uint32_t n0 = b1 ? n[1] : n[0], n1 = b1 ? n[2] : n[1], n2 = b1 ? n[3] : n[2];
-        fn = __funnelshift_r(n0, n1, sn); rn = __funnelshift_r(n1, n2, sn);
-        const uint32_t s0 = b1 ? s[1] : s[0], s1 = b1 ? s[2] : s[1], s2 = b1 ? s[3] : s[2];
-        ls = __funnelshift_r(__funnelshift_r(s0, s1, sn), __funnelshift_r(s1, s2, sn), 12);
+    for (int i = 0; i < NW / 2 + 1; i++) {
+        const uint2 v = *reinterpret_cast<const uint2*>(nb + w0 + 2 * i);
+        x[2 * i] = v.x; x[2 * i + 1] = v.y;
     }
-};
-__device__ __forceinline__ SeqBlock load_block(const uint64_t* __restrict__ pk, const uint32_t* __restrict__ nm, const uint32_t* __restrict__ sm,
-                                               uint32_t first) {
-    SeqBlock b;
-    b.c0 = first & ~63u;
-    const uint32_t w0 = b.c0 >> 5;                                 // even: 16-byte aligned in pk, 8-byte aligned in nm / sm
-    const uint4 a = *reinterpret_cast<const uint4*>(pk + w0), c = *reinterpret_cast<const uint4*>(pk + w0 + 2);
-    b.w[0] = (uint64_t)a.x | ((uint64_t)a.y << 32); b.w[1] = (uint64_t)a.z | ((uint64_t)a.w << 32);
-    b.w[2] = (uint64_t)c.x | ((uint64_t)c.y << 32); b.w[3] = (uint64_t)c.z | ((uint64_t)c.w << 32);
-    const uint2 n0 = *reinterpret_cast<const uint2*>(nm + w0), n1 = *reinterpret_cast<const uint2*>(nm + w0 + 2);
-    b.n[0] = n0.x; b.n[1] = n0.y; b.n[2] = n1.x; b.n[3] = n1.y;
-    if (sm != nm) {                                                // uniform: a genome without lower case hands out nm for both
-        const uint2 s0 = *reinterpret_cast<const uint2*>(sm + w0), s1 = *reinterpret_cast<const uint2*>(sm + w0 + 2);
-        b.s[0] = s0.x; b.s[1] = s0.y; b.s[2] = s1.x; b.s[3] = s1.y;
-    } else {
-        b.s[0] = b.n[0]; b.s[1] = b.n[1]; b.s[2] = b.n[2]; b.s[3] = b.n[3];
-    }
-    return b;
+#pragma unroll
+    for (int m = 0; m < NW; m++) w[m] = __funnelshift_r(odd ? x[m + 1] : x[m], odd ? x[m + 2] : x[m + 1], sh);
+}
+// Leader test on 19 merged columns (l0: columns 0..7, l1: 8..15, l2: 16..18) that hold no non-ACGT base: do they form a seed
+// hit, i.e. x = 0 in every care column, or (transition) x = 2 in exactly one and 0 in the others?
+__device__ __forceinline__ bool seed_match_merged(uint32_t l0, uint32_t l1, uint32_t l2, bool transition) {
+    const uint32_t x0 = l0 & 0x30030333u, x1 = l1 & 0x30303003u, x2 = l2 & 0x333u;   // x bits of the care columns
+    if ((x0 | x1 | x2) == 0) return true;
+    return transition && ((x0 | x1 | x2) & 0x11111111u) == 0 && __popc(x0) + __popc(x1) + __popc(x2) == 1;
 }
 
 // Appends the survivors of a warp (diagonal, query position) at one atomically reserved range of surv.
@@ -224,21 +209,23 @@ constexpr int SC_RING = 128;               // descriptors per warp: < 32 pending
                                            // (a small ring keeps shared memory low, which leaves the SM more L1 for the gathers)
 constexpr int SC_DQ = 64;                  // deferred hits per warp: < 32 queued (drained at 32) + at most 32 from one batch
 
-// Window b >= 1 of the right or the left side of hit (hi, hj) in extension order (the left side reversed), for a lane whose
-// side is still open (D); zero columns (a no-op) otherwise.
+// Window b >= 1 of the right or the left side of hit (hi, hj) in extension order (the left side reversed), prepared, for a lane
+// whose side is still open (D); zero columns (a no-op) otherwise. an: the window holds a non-ACGT column.
 __device__ __forceinline__ void s1_later_window(const GenomeView& T, const GenomeView& Q, uint32_t hi, uint32_t hj, bool right, int b, int D,
-                                                uint64_t& wt, uint64_t& wq, uint32_t& an) {
-    wt = 0; wq = 0; an = 0;
+                                                uint32_t (&w)[4], bool& an) {
+    w[0] = w[1] = w[2] = w[3] = 0; an = false;
     if (D >= S1_DONE / 2) return;
+    const uint32_t d = right ? SEED_SPAN + S1_WINDOW * b : SEED_SPAN - S1_WINDOW * b - 32;
+    uint32_t t[4], q[4];
+    nib_span<4>(T.nb, hi + d, t); nib_span<4>(Q.nb, hj + d, q);
     if (right) {
-        const uint32_t ct = hi + SEED_SPAN + S1_WINDOW * b, cq = hj + SEED_SPAN + S1_WINDOW * b;
-        wt = window32(T.pk, ct); wq = window32(Q.pk, cq);
-        an = (nwindow32(T.nm, ct) | nwindow32(Q.nm, cq)) & S1_WINDOW_MASK;
+#pragma unroll
+        for (int i = 0; i < 4; i++) w[i] = nib_merge(t[i], q[i]);
     } else {
-        const uint32_t ct = hi + SEED_SPAN - S1_WINDOW * b - 32, cq = hj + SEED_SPAN - S1_WINDOW * b - 32;
-        wt = rev2groups(window32(T.pk, ct)); wq = rev2groups(window32(Q.pk, cq));
-        an = __brev(nwindow32(T.nm, ct) | nwindow32(Q.nm, cq)) & S1_WINDOW_MASK;
+#pragma unroll
+        for (int i = 0; i < 4; i++) w[i] = nib_rev(nib_merge(t[3 - i], q[3 - i]));
     }
+    an = s1_prepare(w);
 }
 
 template <int MINB, uint32_t TAILVOTES>
@@ -341,14 +328,14 @@ seed_scan_kernel(GenomeView T, GenomeView Q, const uint32_t* __restrict__ off, c
                 s1_unpack(r.w, best_l, dl);
             }
             dq_head += nd;
-            uint64_t wt, wq; uint32_t an;
+            uint32_t w[4]; bool an;
             if (!__all_sync(0xffffffffu, dr >= S1_DONE / 2)) {
-                s1_later_window(T, Q, hi, hj, true, 1, dr, wt, wq, an);
-                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, wt, wq, an, X, best_r, dr, nchunks);
+                s1_later_window(T, Q, hi, hj, true, 1, dr, w, an);
+                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, w, an, best_r, dr, nchunks);
             }
             if (!__all_sync(0xffffffffu, dl >= S1_DONE / 2)) {
-                s1_later_window(T, Q, hi, hj, false, 2, dl, wt, wq, an);
-                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, wt, wq, an, X, best_l, dl, nchunks);
+                s1_later_window(T, Q, hi, hj, false, 2, dl, w, an);
+                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, w, an, best_l, dl, nchunks);
             }
         } else {
             // ---------------- phase B: one batch of up to 32 hits, one per lane
@@ -374,36 +361,40 @@ seed_scan_kernel(GenomeView T, GenomeView Q, const uint32_t* __restrict__ off, c
                 }
             }
             // Everything the batch needs that does not depend on the x-drop outcome: leader window (p - 1), first right window
-            // (p + 19) and first left window (p - 13). All three lie inside the 128 columns that start at the 64-column boundary
-            // below p - 13, so each sequence is fetched as ONE aligned block (32 bytes of packed bases, 16 of flags: four load
-            // instructions per sequence instead of twelve) and the windows are cut out of registers. After the bank fix of the
-            // extension table (xdrop_table.cuh) the scan is bound by the integer ALU pipe (ncu on C4: alu pipe 74 % busy, L1 data
-            // pipe 65 %, DRAM 11 %; profiles/r2_seed_scan_c4_v2_ncu_summary.txt); taking the pos[] and target gathers of the next
-            // batch off the critical path (a pipelined variant, measured) changed nothing and was dropped.
-            uint64_t lt = 0, lq = 0, rt = 0, rq = 0, ft = 0, fq = 0;
-            uint32_t ln = 1, rn = 0, fn = 0;
+            // (p + 19) and first left window (p - 13). All three lie inside the 64 columns from p - 13: the nb codes of both
+            // sequences there are read with five aligned 8-byte loads each, merged once, and the windows are cut out of the merged
+            // words. After the bank fix of the extension table the scan is bound by the integer ALU pipe (ncu on C4: alu pipe
+            // 74 % busy, L1 data pipe 65 %, DRAM 11 %; profiles/r2_seed_scan_c4_v2_ncu_summary.txt); taking the pos[] and target
+            // gathers of the next batch off the critical path (a pipelined variant, measured) changed nothing and was dropped.
+            uint32_t rw[4] = {0, 0, 0, 0}, fw[4] = {0, 0, 0, 0};
+            bool ra = false, fa = false;
             if (live) {
-                const SeqBlock bt = load_block(T.pk, T.nm, T.sm, hi - 13), bq = load_block(Q.pk, Q.nm, Q.sm, hj - 13);
-                uint32_t tfn, trn, tls, qfn, qrn, qls;
-                bt.windows(hi - 13, ft, lt, rt, tfn, trn, tls);
-                bq.windows(hj - 13, fq, lq, rq, qfn, qrn, qls);
-                ln = (tls | qls) & SEED_WINDOW_MASK19;
-                rn = (trn | qrn) & S1_WINDOW_MASK;
-                fn = __brev(tfn | qfn) & S1_WINDOW_MASK;
+                uint32_t bt[8], bq[8], m[8];
+                nib_span<8>(T.nb, hi - 13, bt); nib_span<8>(Q.nb, hj - 13, bq);
+#pragma unroll
+                for (int i = 0; i < 8; i++) m[i] = nib_merge(bt[i], bq[i]);
+                const uint32_t l0 = __funnelshift_r(m[1], m[2], 16), l1 = __funnelshift_r(m[2], m[3], 16), l2 = m[3] >> 16;
+                // not seedable: a non-ACGT column (bit 3 of the merged code), or a soft-masked one when either genome has lower
+                // case (uniform; such a genome hands out an sm plane of its own)
+                const uint32_t ln = (T.sm != T.nm || Q.sm != Q.nm) ? (nwindow32(T.sm, hi - 1) | nwindow32(Q.sm, hj - 1)) & SEED_WINDOW_MASK19
+                                                                   : ((l0 | l1) & 0x88888888u) | (l2 & 0x888u);
                 // spec D1: only run leaders are candidates
-                if (ln == 0 && seed_match(lt, lq, transition != 0)) live = false; else n_lead++;
+                if (ln == 0 && seed_match_merged(l0, l1, l2, transition != 0)) live = false; else n_lead++;
+#pragma unroll
+                for (int i = 0; i < 4; i++) { rw[i] = m[4 + i]; fw[i] = nib_rev(m[3 - i]); }
+                ra = s1_prepare(rw); fa = s1_prepare(fw);
             }
             // Right of the seed: window 0 of 30 columns. Left, from the last seed column downwards: windows 0 and 1, reversed so
-            // that the same forward-order table applies. The first window of either side comes out of the blocks above and runs
+            // that the same forward-order table applies. The first window of either side comes out of the block above and runs
             // without polling (some lane of 32 is practically always still open at its end; on the left its first 19 columns are
             // the seed itself); left window 1 (needed by ~90 % of hits) is skipped when all lanes are done and polled inside.
             if (live) { dr = S1_D0; dl = S1_D0; }
-            xdrop_window30<0u>(s1tab_sa, s1_m10, s1_m9, rt, rq, rn, X, best_r, dr, nchunks);
-            xdrop_window30<0u>(s1tab_sa, s1_m10, s1_m9, rev2groups(ft), rev2groups(fq), fn, X, best_l, dl, nchunks);
+            xdrop_window30<0u>(s1tab_sa, s1_m10, s1_m9, rw, ra, best_r, dr, nchunks);
+            xdrop_window30<0u>(s1tab_sa, s1_m10, s1_m9, fw, fa, best_l, dl, nchunks);
             if (!__all_sync(0xffffffffu, dl >= S1_DONE / 2)) {
-                uint64_t wt, wq; uint32_t an;
-                s1_later_window(T, Q, hi, hj, false, 1, dl, wt, wq, an);
-                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, wt, wq, an, X, best_l, dl, nchunks);
+                uint32_t w[4]; bool an;
+                s1_later_window(T, Q, hi, hj, false, 1, dl, w, an);
+                xdrop_window30<TAILVOTES>(s1tab_sa, s1_m10, s1_m9, w, an, best_l, dl, nchunks);
             }
             // a hit still open on either side goes to the queue and is decided by a drain, also one whose best_r + best_l already
             // reaches K: stage1_cells counts every chunk a hit is open in

@@ -10,7 +10,10 @@
 // Storage: pk  = 2 bits/base, 32 bases per uint64 word, base p in bits [2(p%32), 2(p%32)+1];
 //          nm  = 1 bit/base, 32 bases per uint32 word, 1 = not A/C/G/T (N, IUPAC, pad): scores -100 in every extension;
 //          sm  = nm | soft-mask: lower-case input is excluded from SEEDING on both sequences, as LASTZ does without
-//                [unmask] (a 19-mer window holding such a base is no seed word), but is extended through by its base.
+//                [unmask] (a 19-mer window holding such a base is no seed word), but is extended through by its base;
+//          nb  = 4 bits/base, 8 bases per uint32 word, base p in bits [4(p%8), 4(p%8)+3]: base | parity << 2 (parity = C or G)
+//                for A/C/G/T, 8 for anything else (N, IUPAC, pad). The seed scan merges a target and a query word of it into one
+//                code per column (seed.cu: nib_merge) that indexes its x-drop table directly.
 #pragma once
 #include "common.cuh"
 
@@ -29,6 +32,7 @@ struct Genome {
     DevBuf<uint32_t> nm;              // G/32 + 2 words
     DevBuf<uint32_t> sm;              // G/32 + 2 words: 1 = not seedable (non-ACGT, pad, or soft-masked = lower case in the input)
     bool has_soft = false;            // false: no lower-case base anywhere, sm == nm bit for bit and kernels are handed nm (one plane to gather from)
+    DevBuf<uint32_t> nb;              // G/8 + 8 words: 4-bit codes (see above)
     DevBuf<uint8_t> codes;            // 1 byte/base for the gapped DP: base | parity << 2, 8 = other, 12 = pad (genome.cu:code_byte)
     DevBuf<uint32_t> d_off, d_len;
     DevBuf<uint32_t> d_nfree;         // per scaffold: 1 = every base is A/C/G/T
@@ -44,6 +48,7 @@ struct GenomeView {   // what kernels receive
     const uint64_t* __restrict__ pk;
     const uint32_t* __restrict__ nm;
     const uint32_t* __restrict__ sm;
+    const uint32_t* __restrict__ nb;
     const uint8_t* __restrict__ codes;
     const uint32_t* __restrict__ off;
     const uint32_t* __restrict__ len;
@@ -51,7 +56,7 @@ struct GenomeView {   // what kernels receive
     int nscaf;
     uint32_t G;
 };
-inline GenomeView view(const Genome& g) { return GenomeView{g.pk.get(), g.nm.get(), g.has_soft ? g.sm.get() : g.nm.get(), g.codes.get(), g.d_off.get(), g.d_len.get(), g.d_nfree.get(), g.nscaf, (uint32_t)g.G}; }
+inline GenomeView view(const Genome& g) { return GenomeView{g.pk.get(), g.nm.get(), g.has_soft ? g.sm.get() : g.nm.get(), g.nb.get(), g.codes.get(), g.d_off.get(), g.d_len.get(), g.d_nfree.get(), g.nscaf, (uint32_t)g.G}; }
 
 // HOXD70 as LASTZ's default, row = target base, col = query base (index t*4+q)
 static __constant__ int c_sub[16] = {91, -114, -31, -123, -114, 100, -125, -31, -31, -125, 100, -114, -123, -31, -114, 91};
@@ -80,25 +85,20 @@ __device__ __forceinline__ uint32_t nwindow32(const uint32_t* __restrict__ nm, u
 // 32 bases ENDING at p (inclusive), base p-c in bits [2c, 2c+1] (i.e. reversed order) is awkward to build;
 // leftward walks instead fetch the aligned window that contains p and index into it.
 
+// nb code of one base (see above)
+__device__ __forceinline__ uint32_t nib_code(uint32_t base, uint32_t bad) {
+    return bad ? 8u : (base | (((base ^ (base >> 1)) & 1u) << 2));
+}
+
 __device__ __forceinline__ int sub_score(uint32_t tb, uint32_t qb, uint32_t anyn) {
     return anyn ? SCORE_N : c_sub[(tb << 2) | qb];
 }
 
 // 12-of-19 spaced seed 1110100110010101111: care offsets {0,1,2,4,7,8,11,13,15,16,17,18}
-constexpr uint64_t SEED_CARE_MASK =
-    (0x3Full) | (0x3ull << 8) | (0xFull << 14) | (0x3ull << 22) | (0x3ull << 26) | (0xFFull << 30);
-constexpr uint64_t SEED_LOW_BITS = 0x5555555555555555ull;
 constexpr uint32_t SEED_WINDOW_MASK19 = (1u << SEED_SPAN) - 1u;
 
 __device__ __forceinline__ uint32_t seed_key(uint64_t w) {
     return (uint32_t)(w & 0x3F) | ((uint32_t)(w >> 8) & 3u) << 6 | ((uint32_t)(w >> 14) & 0xFu) << 8 |
            ((uint32_t)(w >> 22) & 3u) << 12 | ((uint32_t)(w >> 26) & 3u) << 14 | ((uint32_t)(w >> 30) & 0xFFu) << 16;
 }
-// do two clean 19-mer windows form a seed hit (exact on the care positions, or one transition)?
-__device__ __forceinline__ bool seed_match(uint64_t wt, uint64_t wq, bool transition) {
-    const uint64_t x = (wt ^ wq) & SEED_CARE_MASK;
-    if (x == 0) return true;
-    return transition && (x & SEED_LOW_BITS) == 0 && __popcll(x) == 1;
-}
-
 }  // namespace mb2

@@ -1,5 +1,5 @@
-// xdrop_table.cuh -- exact gap-free x-drop at three columns per shared-memory table lookup (used by the first-stage
-// filter of seed.cu and the thread-per-diagonal HSP extension of hsp.cu).
+// xdrop_table.cuh -- exact gap-free x-drop at three columns per shared-memory table lookup (used by the thread-per-diagonal
+// HSP extension of hsp.cu; the first-stage filter of seed.cu has a table of the same size indexed by merged 4-bit codes).
 //
 // Entry for target bases t0 t1 t2 / query bases q0 q1 q2 (index = q6 << 6 | t6, first column in the low bits; the shared-memory
 // bank comes from the TARGET bases: the 32 hits of a seed-scan batch mostly share one query position, so with the query bits in

@@ -60,6 +60,14 @@ class Genome:
         _lib.check(_lib.lib().mb2_genome_decode(self.handle, scaf, out.ctypes.data))
         return out
 
+    def nibbles(self) -> np.ndarray:
+        """Test hook: the 4-bit code of every padded position (uint8 per position, the device plane unpacked)."""
+        n = C.c_uint64(0)
+        _lib.check(_lib.lib().mb2_test_genome_nibbles(self.handle, None, 0, C.byref(n)))
+        words = np.zeros(int(n.value), dtype=np.uint32)
+        _lib.check(_lib.lib().mb2_test_genome_nibbles(self.handle, words.ctypes.data, len(words), C.byref(n)))
+        return ((words[:, None] >> (4 * np.arange(8, dtype=np.uint32))) & 15).astype(np.uint8).reshape(-1)
+
     def close(self):
         if getattr(self, 'handle', None):
             _lib.lib().mb2_genome_free(self.handle)
