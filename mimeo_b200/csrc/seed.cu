@@ -139,14 +139,20 @@ __device__ __forceinline__ void s1_unpack(uint32_t w, int& best, int& D) {
     D = (w >> 16) == 0xFFFFu ? S1_DONE : (int)(w >> 16);
 }
 
-// Merged code of target and query nb words (see s1_entry): one LOP3
+// Merged code of target and query nb words (see s1_entry): M ? t ^ q : t | q with M = 0x33333333, one LOP3 (LUT 0x7A for
+// the operands t, M, q; written out because ptxas splits the plain expression into three)
 __device__ __forceinline__ uint32_t nib_merge(uint32_t t, uint32_t q) {
-    return ((t ^ q) & 0x33333333u) | ((t | q) & 0xCCCCCCCCu);
+    uint32_t m;
+    asm("lop3.b32 %0, %1, %2, %3, 0x7A;" : "=r"(m) : "r"(t), "r"(0x33333333u), "r"(q));
+    return m;
 }
-// the eight 4-bit groups of a word in reverse order
+// the eight 4-bit groups of a word in reverse order: a byte reversal, then M ? x >> 4 : x << 4 with M = 0x0F0F0F0F (LUT 0xE2
+// for the operands x >> 4, M, x << 4)
 __device__ __forceinline__ uint32_t nib_rev(uint32_t x) {
     x = __byte_perm(x, 0u, 0x0123u);
-    return ((x >> 4) & 0x0F0F0F0Fu) | ((x << 4) & 0xF0F0F0F0u);
+    uint32_t r;
+    asm("lop3.b32 %0, %1, %2, %3, 0xE2;" : "=r"(r) : "r"(x >> 4), "r"(0x0F0F0F0Fu), "r"(x << 4));
+    return r;
 }
 // NW words of nb codes = the 8 NW columns from column p (p in the low bits of w[0]), read as NW / 2 + 1 aligned 8-byte loads
 template <int NW>
