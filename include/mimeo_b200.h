@@ -310,6 +310,24 @@ MB2_API int mb2_tandem_mask_runs(const mb2_genome* g, const int32_t* scaf, const
 MB2_API int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
                                  const mb2_tandem_params* p, uint64_t store_budget, uint64_t* masked, mb2_tandem_runs* runs);
 MB2_API void mb2_free_tandem_runs(mb2_tandem_runs* r);
+/* The tandem-repeat report of `--reportTRF` (DESIGN §2, R1-R6; not TRF's .dat): mb2_tandem_mask_runs, and in the same call
+ * one entry per run r of `runs` (span order, runs ascending) describing the tandem array in that run: period (R2), score
+ * (R6, may be negative), matches to the consensus (R4), count[4r .. 4r+3] of A, C, G, T (R5), and the consensus (R3),
+ * consensus[cons_off[r] .. cons_off[r+1]), period[r] bytes of A/C/G/T/N without a terminator. Identical runs are computed
+ * once. Arrays owned by the library; free rep with mb2_free_tandem_report and runs with mb2_free_tandem_runs (both also
+ * after an error). Parameter checks are mb2_tandem_mask's. */
+typedef struct mb2_tandem_repeats {
+    int32_t* period;
+    int64_t* score;
+    uint64_t* matches;
+    uint64_t* count;     /* 4 per run */
+    uint64_t* cons_off;  /* n + 1 entries */
+    char* consensus;
+    uint64_t n;          /* number of runs */
+} mb2_tandem_repeats;
+MB2_API int mb2_tandem_report(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                              const mb2_tandem_params* p, uint64_t* masked, mb2_tandem_runs* runs, mb2_tandem_repeats* rep);
+MB2_API void mb2_free_tandem_report(mb2_tandem_repeats* r);
 
 /* ---- device primitives exposed for parity tests ------------------------------------------- */
 /* Stable LSD radix sort of HOST arrays on bits [begin_bit, end_bit) (vals may be NULL). */

@@ -64,6 +64,11 @@ class TandemRuns(C.Structure):
     _fields_ = [('off', c_u64p), ('start', c_i64p), ('end', c_i64p), ('n', C.c_uint64)]
 
 
+class TandemRepeats(C.Structure):
+    _fields_ = [('period', c_i32p), ('score', c_i64p), ('matches', c_u64p), ('count', c_u64p), ('cons_off', c_u64p),
+                ('consensus', C.c_void_p), ('n', C.c_uint64)]
+
+
 class Segments(C.Structure):
     _fields_ = [('chrom', c_i32p), ('start', c_i32p), ('end', c_i32p), ('n', C.c_uint64), ('on_device', C.c_int)]
 
@@ -126,6 +131,9 @@ SIGNATURES = {
     'mb2_test_tandem_mask': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(TandemParams), C.c_uint64,
                                        C.c_void_p, C.POINTER(TandemRuns)]),
     'mb2_free_tandem_runs': (None, [C.POINTER(TandemRuns)]),
+    'mb2_tandem_report': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(TandemParams), C.c_void_p,
+                                    C.POINTER(TandemRuns), C.POINTER(TandemRepeats)]),
+    'mb2_free_tandem_report': (None, [C.POINTER(TandemRepeats)]),
     'mb2_test_sort_u32': (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int]),
     'mb2_test_sort_u64': (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int]),
     'mb2_test_sort_u32_pair': (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int]),

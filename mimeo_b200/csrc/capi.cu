@@ -593,6 +593,24 @@ int mb2_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t* sta
         tandem_mask(*g->g, scaf, start, len, n, to_tandem(p), 0, masked, nullptr);
     });
 }
+// copies the merged runs of every span into the library-owned arrays of `runs`
+static void fill_runs(const std::vector<std::vector<std::pair<int64_t, int64_t>>>& iv, uint64_t n, mb2_tandem_runs* runs) {
+    size_t total = 0;
+    for (const auto& v : iv) total += v.size();
+    runs->off = (uint64_t*)malloc((n + 1) * sizeof(uint64_t));
+    runs->start = (int64_t*)malloc((total ? total : 1) * sizeof(int64_t));
+    runs->end = (int64_t*)malloc((total ? total : 1) * sizeof(int64_t));
+    MB2_REQUIRE(runs->off && runs->start && runs->end, MB2_ERR_INTERNAL, "tandem_mask_runs: host allocation failed");
+    runs->n = n;
+    runs->off[0] = 0;
+    for (uint64_t k = 0; k < n; k++) {
+        for (size_t t = 0; t < iv[k].size(); t++) {
+            runs->start[runs->off[k] + t] = iv[k][t].first;
+            runs->end[runs->off[k] + t] = iv[k][t].second;
+        }
+        runs->off[k + 1] = runs->off[k] + iv[k].size();
+    }
+}
 static int tandem_mask_runs(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
                             const mb2_tandem_params* p, uint64_t store_budget, uint64_t* masked, mb2_tandem_runs* runs) {
     return guarded([&] {
@@ -600,21 +618,7 @@ static int tandem_mask_runs(const mb2_genome* g, const int32_t* scaf, const int6
         std::memset(runs, 0, sizeof(*runs));
         std::vector<std::vector<std::pair<int64_t, int64_t>>> iv;
         tandem_mask(*g->g, scaf, start, len, n, to_tandem(p), (size_t)store_budget, masked, &iv);
-        size_t total = 0;
-        for (const auto& v : iv) total += v.size();
-        runs->off = (uint64_t*)malloc((n + 1) * sizeof(uint64_t));
-        runs->start = (int64_t*)malloc((total ? total : 1) * sizeof(int64_t));
-        runs->end = (int64_t*)malloc((total ? total : 1) * sizeof(int64_t));
-        MB2_REQUIRE(runs->off && runs->start && runs->end, MB2_ERR_INTERNAL, "tandem_mask_runs: host allocation failed");
-        runs->n = n;
-        runs->off[0] = 0;
-        for (uint64_t k = 0; k < n; k++) {
-            for (size_t t = 0; t < iv[k].size(); t++) {
-                runs->start[runs->off[k] + t] = iv[k][t].first;
-                runs->end[runs->off[k] + t] = iv[k][t].second;
-            }
-            runs->off[k + 1] = runs->off[k] + iv[k].size();
-        }
+        fill_runs(iv, n, runs);
     });
 }
 int mb2_tandem_mask_runs(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
@@ -628,6 +632,39 @@ int mb2_test_tandem_mask(const mb2_genome* g, const int32_t* scaf, const int64_t
 void mb2_free_tandem_runs(mb2_tandem_runs* r) {
     if (!r) return;
     free(r->off); free(r->start); free(r->end);
+    std::memset(r, 0, sizeof(*r));
+}
+int mb2_tandem_report(const mb2_genome* g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n,
+                      const mb2_tandem_params* p, uint64_t* masked, mb2_tandem_runs* runs, mb2_tandem_repeats* rep) {
+    return guarded([&] {
+        MB2_REQUIRE(g && g->g && runs && rep, MB2_ERR_INVALID_ARG, "tandem_report: null argument");
+        std::memset(runs, 0, sizeof(*runs));
+        std::memset(rep, 0, sizeof(*rep));
+        std::vector<std::vector<std::pair<int64_t, int64_t>>> iv;
+        TandemReport tr;
+        tandem_report(*g->g, scaf, start, len, n, to_tandem(p), masked, iv, tr);
+        fill_runs(iv, n, runs);
+        const size_t nr = tr.period.size();
+        rep->period = (int32_t*)malloc((nr ? nr : 1) * sizeof(int32_t));
+        rep->score = (int64_t*)malloc((nr ? nr : 1) * sizeof(int64_t));
+        rep->matches = (uint64_t*)malloc((nr ? nr : 1) * sizeof(uint64_t));
+        rep->count = (uint64_t*)malloc((nr ? 4 * nr : 1) * sizeof(uint64_t));
+        rep->cons_off = (uint64_t*)malloc((nr + 1) * sizeof(uint64_t));
+        rep->consensus = (char*)malloc(tr.consensus.size() + 1);
+        MB2_REQUIRE(rep->period && rep->score && rep->matches && rep->count && rep->cons_off && rep->consensus, MB2_ERR_INTERNAL,
+                    "tandem_report: host allocation failed");
+        rep->n = nr;
+        std::copy(tr.period.begin(), tr.period.end(), rep->period);
+        std::copy(tr.score.begin(), tr.score.end(), rep->score);
+        std::copy(tr.matches.begin(), tr.matches.end(), rep->matches);
+        std::copy(tr.count.begin(), tr.count.end(), rep->count);
+        std::copy(tr.cons_off.begin(), tr.cons_off.end(), rep->cons_off);
+        std::copy(tr.consensus.begin(), tr.consensus.end(), rep->consensus);
+    });
+}
+void mb2_free_tandem_report(mb2_tandem_repeats* r) {
+    if (!r) return;
+    free(r->period); free(r->score); free(r->matches); free(r->count); free(r->cons_off); free(r->consensus);
     std::memset(r, 0, sizeof(*r));
 }
 

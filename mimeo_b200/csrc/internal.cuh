@@ -142,6 +142,16 @@ uint64_t format_segment_gff(const int32_t* chrom, const int32_t* start, const in
 struct TandemParams { int match = 2, mismatch = 7, delta = 7, minscore = 50, maxperiod = 50; };
 void tandem_mask(const Genome& g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n, const TandemParams& p,
                  size_t store_budget, uint64_t* masked, std::vector<std::vector<std::pair<int64_t, int64_t>>>* intervals);
+// the report of `--reportTRF` (DESIGN §2, R1-R6): tandem_mask with intervals, then one row per run of every span, in span
+// order and ascending within a span; row r's consensus is consensus[cons_off[r], cons_off[r+1])
+struct TandemReport {
+    std::vector<int32_t> period;
+    std::vector<int64_t> score;
+    std::vector<uint64_t> matches, count, cons_off;    // count: 4 per row (A, C, G, T); cons_off: rows + 1
+    std::string consensus;
+};
+void tandem_report(const Genome& g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n, const TandemParams& p,
+                   uint64_t* masked, std::vector<std::vector<std::pair<int64_t, int64_t>>>& intervals, TandemReport& rep);
 
 // counters layout (device, unsigned long long[16])
 enum { CNT_SURV = 0, CNT_SEED_HITS = 1, CNT_LEADERS = 2, CNT_S1_CELLS = 3, CNT_HSPS = 4, CNT_EXTENDED = 5, CNT_S2_CELLS = 6,

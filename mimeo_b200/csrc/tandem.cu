@@ -1,11 +1,14 @@
 // tandem.cu -- the tandem-repeat mask of `mimeo map --maxtandem` (DESIGN §2 T1-T4, kernel in tandem_warp.cuh): span
-// validation, dedupe, scheduling (one warp per distinct span, longest first) and the storage bound.
+// validation, dedupe, scheduling (one warp per distinct span, longest first) and the storage bound; and the report of
+// `--reportTRF` on the masked runs (DESIGN §2 R1-R6, kernel in tandem_report_warp.cuh), with the same scheduling per
+// distinct run.
 #include <algorithm>
 #include <numeric>
 #include <tuple>
 
 #include "internal.cuh"
 #include "seq.cuh"
+#include "tandem_report_warp.cuh"
 #include "tandem_warp.cuh"
 #include "mimeo_b200.h"
 
@@ -110,6 +113,20 @@ void run_layout(const Genome& g, const std::vector<uint64_t>& ugs, const std::ve
         b0 = b1;
     }
 }
+template <int NT>
+__global__ void __launch_bounds__(WARPS * 32) tandem_report_kernel(const uint8_t* __restrict__ codes, const uint64_t* __restrict__ gstart,
+                                                                   const int32_t* __restrict__ len, uint32_t nruns, tr::Params p,
+                                                                   tr::Out o, uint32_t* next) {
+    __shared__ tr::Scratch sh[WARPS];
+    const int w = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (;;) {
+        uint32_t k = 0;
+        if (lane == 0) k = atomicAdd(next, 1u);
+        k = __shfl_sync(0xffffffffu, k, 0);
+        if (k >= nruns) break;
+        tr::report_warp<NT>(codes + gstart[k], len[k], p, sh[w], o, k);
+    }
+}
 }  // namespace
 
 void tandem_mask(const Genome& g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n, const TandemParams& tp,
@@ -169,6 +186,86 @@ void tandem_mask(const Genome& g, const int32_t* scaf, const int64_t* start, con
     for (uint64_t k = 0; k < n; k++) {
         masked[k] = um[uof[k]];
         if (intervals) (*intervals)[k] = uiv[uof[k]];
+    }
+}
+
+void tandem_report(const Genome& g, const int32_t* scaf, const int64_t* start, const int64_t* len, uint64_t n, const TandemParams& tp,
+                   uint64_t* masked, std::vector<std::vector<std::pair<int64_t, int64_t>>>& intervals, TandemReport& rep) {
+    tandem_mask(g, scaf, start, len, n, tp, 0, masked, &intervals);
+    // rows = runs in span order; distinct runs by (genome offset, length), longest first
+    std::vector<std::pair<uint64_t, int32_t>> key;
+    for (uint64_t k = 0; k < n; k++)
+        for (const auto& r : intervals[k]) {
+            MB2_REQUIRE(r.second - r.first >= 1, MB2_ERR_INTERNAL, "tandem_report: masked run shorter than 2");
+            key.emplace_back((uint64_t)g.off[scaf[k]] + (uint64_t)(start[k] + r.first), (int32_t)(r.second - r.first + 1));
+        }
+    const size_t nrow = key.size();
+    std::vector<size_t> idx(nrow);
+    std::iota(idx.begin(), idx.end(), 0);
+    std::sort(idx.begin(), idx.end(), [&](size_t a, size_t b) { return key[a] < key[b]; });
+    std::vector<uint64_t> ugs;
+    std::vector<int32_t> ulen;
+    std::vector<size_t> uof(nrow);
+    for (size_t x = 0; x < nrow; x++) {
+        if (x == 0 || key[idx[x]] != key[idx[x - 1]]) { ugs.push_back(key[idx[x]].first); ulen.push_back(key[idx[x]].second); }
+        uof[idx[x]] = ugs.size() - 1;
+    }
+    const size_t nu = ugs.size();
+    std::vector<size_t> order(nu);
+    std::iota(order.begin(), order.end(), 0);
+    std::stable_sort(order.begin(), order.end(), [&](size_t a, size_t b) { return ulen[a] > ulen[b]; });
+    std::vector<uint64_t> gs(nu), coff(nu + 1, 0);
+    std::vector<int32_t> ln(nu);
+    for (size_t x = 0; x < nu; x++) {
+        gs[x] = ugs[order[x]];
+        ln[x] = ulen[order[x]];
+        coff[x + 1] = coff[x] + (uint64_t)std::min(tp.maxperiod, ln[x] - 1);
+    }
+    std::vector<int32_t> per(nu);
+    std::vector<int64_t> sc(nu);
+    std::vector<uint64_t> mt(nu), cnt(4 * nu);
+    std::string cons(coff[nu], 'N');
+    if (nu) {
+        ensure_init();
+        cudaStream_t s = ctx().stream;
+        DevBuf<uint64_t> d_gs(nu), d_coff(nu), d_mt(nu), d_cnt(4 * nu);
+        DevBuf<int32_t> d_len(nu), d_per(nu);
+        DevBuf<int64_t> d_sc(nu);
+        DevBuf<char> d_cons(coff[nu]);
+        DevBuf<uint32_t> d_next(1);
+        MB2_CUDA(cudaMemcpyAsync(d_gs.get(), gs.data(), nu * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+        MB2_CUDA(cudaMemcpyAsync(d_coff.get(), coff.data(), nu * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
+        MB2_CUDA(cudaMemcpyAsync(d_len.get(), ln.data(), nu * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        MB2_CUDA(cudaMemsetAsync(d_next.get(), 0, sizeof(uint32_t), s));
+        const tr::Params p{tp.match, tp.mismatch, tp.maxperiod};
+        const unsigned blocks = std::min<unsigned>(cdiv(nu, WARPS), (unsigned)ctx().sm_count * 16u);
+        {
+            ProfScope prof("tandem_report");
+            auto* kernel = tp.maxperiod <= 32 ? tandem_report_kernel<1> : tp.maxperiod <= 64 ? tandem_report_kernel<2>
+                         : tp.maxperiod <= 128 ? tandem_report_kernel<4> : tandem_report_kernel<8>;
+            const tr::Out o{d_per.get(), d_sc.get(), d_mt.get(), d_cnt.get(), d_coff.get(), d_cons.get()};
+            launch(kernel, dim3(blocks), dim3(WARPS * 32), 0, g.codes.get(), d_gs.get(), d_len.get(), (uint32_t)nu, p, o, d_next.get());
+        }
+        MB2_CUDA(cudaMemcpyAsync(per.data(), d_per.get(), nu * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        MB2_CUDA(cudaMemcpyAsync(sc.data(), d_sc.get(), nu * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+        MB2_CUDA(cudaMemcpyAsync(mt.data(), d_mt.get(), nu * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+        MB2_CUDA(cudaMemcpyAsync(cnt.data(), d_cnt.get(), 4 * nu * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+        MB2_CUDA(cudaMemcpyAsync(&cons[0], d_cons.get(), coff[nu], cudaMemcpyDeviceToHost, s));
+        MB2_CUDA(cudaStreamSynchronize(s));
+    }
+    std::vector<size_t> slot(nu);                      // distinct run -> its launch slot
+    for (size_t x = 0; x < nu; x++) slot[order[x]] = x;
+    rep = TandemReport{};
+    rep.cons_off.push_back(0);
+    for (size_t r = 0; r < nrow; r++) {
+        const size_t x = slot[uof[r]];
+        MB2_REQUIRE(per[x] >= 1 && per[x] <= ln[x] - 1 && per[x] <= tp.maxperiod, MB2_ERR_INTERNAL, "tandem_report: period out of range");
+        rep.period.push_back(per[x]);
+        rep.score.push_back(sc[x]);
+        rep.matches.push_back(mt[x]);
+        for (int b = 0; b < 4; b++) rep.count.push_back(cnt[4 * x + b]);
+        rep.consensus.append(cons, coff[x], (size_t)per[x]);
+        rep.cons_off.push_back(rep.consensus.size());
     }
 }
 

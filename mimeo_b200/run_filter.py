@@ -3,7 +3,8 @@ run_filter / trfFasta step, SURVEY 2.1 and 3.5: SSR filtering of repeat librarie
 `self` output). The reference's CLI is not in the tree; this one reuses `mimeo map`'s --t* options, and every record is masked
 as a whole on the GPU under this project's own statement (DESIGN §2, T1-T4), not Tandem Repeats Finder: --TRFpath, --tPM and
 --tPI are accepted and have no effect. --writeTRF also writes every record with its masked positions replaced by N to
-`<outfile without .fa/.fasta/.fna>_TRFmasked.fa`."""
+`<outfile without .fa/.fasta/.fna>_TRFmasked.fa`. --reportTRF writes the period, copy number, consensus, purity and
+composition of every masked run to `<outfile without .fa/.fasta/.fna>_TRF.gff3` (DESIGN §2, R1-R6)."""
 import argparse
 import logging
 import os
@@ -33,6 +34,8 @@ def mainArgs() -> argparse.Namespace:
                         help='Max percentage of a sequence which may be masked as tandem repeat (0..100; 0 drops any sequence with a masked base).')
     parser.add_argument('--writeTRF', action='store_true', default=False,
                         help='Also write every input sequence with its masked positions replaced by N.')
+    parser.add_argument('--reportTRF', action='store_true', default=False,
+                        help='Also write a GFF3 report of every masked tandem array: period, copies, consensus, purity, composition.')
     add_loglevel(parser)
     return parser.parse_args()
 
@@ -59,5 +62,6 @@ def main() -> None:
     else:
         outdir = os.getcwd()
     outfile = os.path.join(outdir, args.outfile)
-    tandem.write_filtered_fasta(records, outfile, args.maxtandem, tparams, tandem.masked_fasta_path(outfile) if args.writeTRF else None)
+    tandem.write_filtered_fasta(records, outfile, args.maxtandem, tparams, tandem.masked_fasta_path(outfile) if args.writeTRF else None,
+                                tandem.fasta_report_path(outfile) if args.reportTRF else None)
     logging.info('Finished!')

@@ -2,7 +2,9 @@
 that percentage are dropped after numbering (import_Align -> tandem filter -> GFF3, SURVEY 3.3), so the surviving rows
 keep their IDs. The mask is this project's own GPU statement (DESIGN §2, T1-T4), not Tandem Repeats Finder: --TRFpath,
 --tPM and --tPI are accepted and have no effect. --writeTRF (with --maxtandem) also writes the .tab lines of the surviving
-hits to `<outfile without .tab>_TRFfiltered.tab`. The same mask filters whole FASTA records in `mimeo filter` (run_filter.py)."""
+hits to `<outfile without .tab>_TRFfiltered.tab`, and --reportTRF (with --maxtandem) the period, copy number, consensus, purity
+and composition of every masked run of every hit evaluated to `<outfile without .tab>_TRF.gff3` (DESIGN §2, R1-R6). The same
+mask filters whole FASTA records in `mimeo filter` (run_filter.py)."""
 import argparse
 import logging
 import os
@@ -46,6 +48,8 @@ def mainArgs() -> argparse.Namespace:
     parser.add_argument('--tmaxperiod', type=int, default=50, help='Tandem mask maximum period (1..256)')
     parser.add_argument('--maxtandem', type=float, default=None, help='Max percentage of an A-genome alignment which may be masked as tandem repeat.')
     parser.add_argument('--writeTRF', action='store_true', default=False, help='With --maxtandem, also write the alignments that pass the filter.')
+    parser.add_argument('--reportTRF', action='store_true', default=False,
+                        help='With --maxtandem, also write a GFF3 report of every masked tandem array of the A-genome spans.')
     add_loglevel(parser)
     return parser.parse_args()
 
@@ -57,6 +61,8 @@ def main() -> None:
     tparams = None
     if args.maxtandem:
         tparams = tandem.params(args.tmatch, args.tmismatch, args.tdelta, args.tminscore, args.tmaxperiod)
+    elif args.reportTRF:
+        logging.warning('--reportTRF works only together with --maxtandem; no tandem repeat report is written.')
     adir_path, bdir_path, outdir, outtab, gffout, tempdir = set_paths(
         adir=args.adir, bdir=args.bdir, afasta=args.afasta, bfasta=args.bfasta, outdir=args.outdir, outtab=args.outfile,
         gffout=args.gffout, runtrf=args.maxtandem)
@@ -81,7 +87,8 @@ def main() -> None:
             logging.warning('No alignments found in %s' % outtab)
             sys.exit(1)
         tandem.write_filtered_map(outtab, body, gffout, chrLens, adir_path, args.maxtandem, tparams,
-                                  tandem.trf_path(outtab) if args.writeTRF else None)
+                                  tandem.trf_path(outtab) if args.writeTRF else None,
+                                  tandem.map_report_path(outtab) if args.reportTRF else None)
     if tempdir and os.path.isdir(tempdir) and not args.keeptemp:
         shutil.rmtree(tempdir)
     logging.info('Finished!')

@@ -6,7 +6,9 @@ One command, one JSON document (stdout and --out), at default mask parameters an
 max SM clock; records, bases and strip cells (2 * sum over records of the cells of one pass); end-to-end wall time of
 `run_filter.main` (FASTA on disk -> files written) with and without --writeTRF; the `tandem_mask` kernel time from mb2_prof
 (separate runs) with and without runs, GCUPS; the longest record alone and its share; records dropped; the C oracle on a
-sample of records plus the longest one, and whether every masked count and run of the sample agrees.
+sample of records plus the longest one, and whether every masked count and run of the sample agrees. The `--reportTRF` leg:
+end-to-end wall time with --reportTRF, the `tandem_report` kernel time next to `tandem_mask` in the same call and its share,
+and whether the counts equal the mask's and every run's report of the sample equals the report oracle.
 
     python scripts/bench_filter.py --steps 3 --warmup 1 --out profiles/r5_filter_library.json
 """
@@ -64,6 +66,7 @@ def main():
     from mimeo_b200 import _lib, run_filter, tandem
     from mimeo_b200.fasta import write_fasta_record
     from oracle import tandem_oracle as to
+    from tests import tandem_report_reference as trr
     smi = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'], capture_output=True, text=True)
     card = smi.stdout.strip().splitlines()[0] if smi.returncode == 0 and smi.stdout.strip() else torch.cuda.get_device_name(0)
     t0 = time.perf_counter()
@@ -86,7 +89,7 @@ def main():
                 write_fasta_record(f, h, s, width=80)
         res['input_fasta_bytes'] = os.path.getsize(infile)
         _lib.init()
-        for key, extra in (('e2e_ms', []), ('e2e_writetrf_ms', ['--writeTRF'])):
+        for key, extra in (('e2e_ms', []), ('e2e_writetrf_ms', ['--writeTRF']), ('e2e_reporttrf_ms', ['--reportTRF'])):
             wall = []
             for k in range(args.warmup + args.steps):
                 sys.argv = ['mimeo-filter', '--infile', infile, '-d', os.path.join(tmp, 'out'), '--loglevel', 'WARNING'] + extra
@@ -117,6 +120,14 @@ def main():
     (m_runs, runs), res['tandem_mask_runs_kernel_ms'], _ = kernel_ms(seqs, True)
     li = int(np.argmax(lens))
     _, res['longest_record_kernel_ms'], _ = kernel_ms([seqs[li]], False)
+    res['report_call_tandem_mask_kernel_ms'], res['tandem_report_kernel_ms'] = [], []
+    for k in range(args.warmup + args.steps):
+        _lib.prof_reset()
+        m_rep, reps = tandem.record_reports(seqs, p)
+        _lib.sync()
+        if k >= args.warmup:
+            res['report_call_tandem_mask_kernel_ms'].append(_lib.prof_get('tandem_mask')[0])
+            res['tandem_report_kernel_ms'].append(_lib.prof_get('tandem_report')[0])
     _lib.prof_enable(False)
     kmed = float(np.median(res['tandem_mask_kernel_ms']))
     res['gcups_kernel_median'] = res['cells_both_passes'] / (kmed * 1e-3) / 1e9
@@ -125,6 +136,9 @@ def main():
     res['records_dropped'] = int(drop.sum())
     res['masked_bp'] = int(m.sum())
     res['counts_equal_with_and_without_runs'] = bool((m == m_runs).all())
+    res['report_runs'] = int(sum(len(rr) for rr in reps))
+    res['report_kernel_over_mask_kernel'] = float(np.median(res['tandem_report_kernel_ms'])) / float(np.median(res['report_call_tandem_mask_kernel_ms']))
+    res['e2e_reporttrf_over_e2e'] = float(np.median(res['e2e_reporttrf_ms'])) / float(np.median(res['e2e_ms']))
     # the C oracle on a sample of records plus the longest one, single-threaded
     rng = np.random.default_rng(7)
     sample = sorted(set(rng.choice(len(recs), args.sample, replace=False).tolist()) | {li})
@@ -135,6 +149,9 @@ def main():
     res['oracle_s_single_thread'] = time.perf_counter() - t0
     res['oracle_sample_cells'] = 2 * strip_cells(lens[sample], p['maxperiod'])
     res['gpu_matches_oracle_on_sample'] = all((int(m[k]), runs[k]) == want[k] for k in sample)
+    res['report_gpu_matches_oracle_on_sample'] = bool((m_rep == m).all()) and all(
+        [(r.start, r.end) for r in reps[k]] == runs[k] and all(trr.report(seqs[k][r.start:r.end + 1], **p) == tuple(r[2:]) for r in reps[k])
+        for k in sample)
     res['records_kept_in_outfile_matches'] = res['records_kept_in_outfile'] == len(recs) - res['records_dropped']
     txt = json.dumps(res, indent=1)
     print(txt)
@@ -143,6 +160,7 @@ def main():
         with open(args.out, 'w') as f:
             f.write(txt + '\n')
     assert res['gpu_matches_oracle_on_sample'] and res['counts_equal_with_and_without_runs'], 'GPU mask differs from the oracle'
+    assert res['report_gpu_matches_oracle_on_sample'], 'GPU tandem report differs from the oracle'
 
 
 if __name__ == '__main__':

@@ -4,7 +4,9 @@ with microsatellites planted in A before B is derived from it, so that the filte
 One command, one JSON document (stdout and --out): card name and power limit; the map step (alignment + device filter)
 and the mask per step with CUDA events (`tandem_mask` tag) after a warm-up; cells (2 * sum of strip cells over distinct
 spans), GCUPS, spans, distinct spans, rows dropped at --maxtandem; the longest span alone; the C oracle on the same spans
-and whether every masked count agrees.
+and whether every masked count agrees. The `--reportTRF` leg: the call that computes the mask and the report together
+(`tandem_report` tag next to `tandem_mask`), the report kernel's share of the mask kernel, and whether its counts equal the
+mask's and every run's report equals the report oracle (tests/tandem_report_oracle.c).
 
     python scripts/bench_tandem.py --steps 5 --warmup 1 --out profiles/r4_tandem_c3.json
 """
@@ -67,6 +69,7 @@ def main():
     from mimeo_b200 import _lib, align as A, tandem
     from mimeo_b200.genome import Genome, align_params
     from oracle import tandem_oracle as to
+    from tests import tandem_report_reference as trr
     smi = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit,clocks.max.sm', '--format=csv,noheader'], capture_output=True, text=True)
     card = smi.stdout.strip().splitlines()[0] if smi.returncode == 0 and smi.stdout.strip() else torch.cuda.get_device_name(0)
     a, b = c3_with_microsatellites()
@@ -113,6 +116,21 @@ def main():
         return m, wall, kern
 
     m, wall, kern = timed(scaf, start0, length, args.steps, args.warmup)
+    rwall, rmask, rkern = [], [], []
+    for k in range(args.warmup + args.steps):
+        _lib.prof_reset()
+        _lib.sync()
+        t0 = time.perf_counter()
+        rm, reps = tandem.masked_reports(T, scaf, start0, length, p)
+        _lib.sync()
+        if k >= args.warmup:
+            rwall.append(1e3 * (time.perf_counter() - t0))
+            rmask.append(_lib.prof_get('tandem_mask')[0])
+            rkern.append(_lib.prof_get('tandem_report')[0])
+    runs = {(c, s + r.start, r.end - r.start + 1): tuple(r[2:]) for c, s, rr in zip(scaf.tolist(), start0.tolist(), reps) for r in rr}
+    t0 = time.perf_counter()
+    rep_agree = bool((rm == m).all()) and all(trr.report(a[an[c]][x:x + n], **p) == v for (c, x, n), v in runs.items())
+    t_rep_oracle = time.perf_counter() - t0
     drop = 100.0 * m.astype(np.float64) / length > args.maxtandem
     L = int(length.max())
     li = int(np.argmax(length))
@@ -139,6 +157,13 @@ def main():
         'longest_span_bp': L, 'longest_span_kernel_ms': lkern, 'longest_span_call_ms': lwall,
         'oracle_s_single_thread': t_oracle, 'oracle_cells_per_s': cells / t_oracle,
         'gpu_matches_oracle': bool(agree),
+        'report_runs': int(sum(len(rr) for rr in reps)), 'report_distinct_runs': len(runs),
+        'report_distinct_run_bp': int(sum(n for _c, _x, n in runs)),
+        'report_call_ms': rwall, 'report_call_tandem_mask_kernel_ms': rmask, 'tandem_report_kernel_ms': rkern,
+        'report_kernel_over_mask_kernel': float(np.median(rkern)) / float(np.median(rmask)),
+        'report_call_over_mask_call': float(np.median(rwall)) / float(np.median(wall)),
+        'report_oracle_s_single_thread': t_rep_oracle,
+        'report_gpu_matches_oracle': rep_agree,
     }
     txt = json.dumps(res, indent=1)
     print(txt)
@@ -148,6 +173,7 @@ def main():
             f.write(txt + '\n')
     T.close(); Q.close()
     assert agree, 'GPU mask differs from the oracle'
+    assert rep_agree, 'GPU tandem report differs from the oracle'
 
 
 if __name__ == '__main__':
